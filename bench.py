@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the north-star path: Router::matches for a batch of PUBLISH topics at 10 M subscriptions.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl own|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl own|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (tokenise -> trie walk -> per-topic match lists) over one batch of
 synthetic topics (workload C3 of BASELINE.json: 10 M subscriptions, 30 % '+', 5 % '#', 6-level IoT topics,
@@ -47,7 +47,13 @@ def _args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=None)
     ap.add_argument("--no-c4", action="store_true", help="skip the retained-tree (config C4) leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the match lists of the last timed step (a fixed sample of its topics, rank 0) "
+                         "as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "own":
+        ap.error("--dump-outputs writes what the own arm's timed path computed; use it with --impl own")
+    return a
 
 
 def _peaks():
@@ -122,6 +128,28 @@ def _workload_desc(cfg, world):
             f"{cfg.n_topics}-topic uniform batch per GPU, seed {cfg.seed:#x}"
             + (f", subscriptions sharded by topic-root hash over {world} GPUs (root-wildcards replicated)" if world > 1 else "")
             + "; L2: the device tables (GBs) and the rotated distinct batches are far larger than the 126 MB L2, no flush between steps")
+
+
+_DUMP_TOPICS = 1 << 16             # topics of the batch that --dump-outputs samples
+_DUMP_BYTES = 60 << 20             # array bytes of one dump: with the .npy headers it stays under 64 MB
+
+
+def _dump_outputs(out_dir, spans, ids, status):
+    """--dump-outputs: one step's match lists (spans uint32[n, 2], ids uint32[], status int32[n]) in a form in which two builds
+    compare equal when they match alike.  The topics are a fixed seeded sample of the batch (all of it when it is small), each
+    topic's ids are sorted (the kernels leave them in any order), and everything is float64, which holds every u32 id exactly.
+    Files: topics (index in the batch), status, counts (-1 for an invalid topic) and ids (concatenated in topic order)."""
+    from rmqtt_b200.engine import MatchResult
+    n = len(spans)
+    topics = np.arange(n) if n <= _DUMP_TOPICS else np.sort(np.random.default_rng(0).choice(n, _DUMP_TOPICS, replace=False))
+    counts, sorted_ids = MatchResult(spans[topics], ids, status[topics], len(ids)).canonical()
+    # the longest prefix of the sample whose topic, status, count and ids fit the byte budget
+    keep = int(np.searchsorted(np.cumsum(3 + np.maximum(counts, 0)), _DUMP_BYTES // 8, side="right"))
+    arrays = {"topics": topics[:keep], "status": status[topics[:keep]], "counts": counts[:keep],
+              "ids": sorted_ids[:int(np.maximum(counts[:keep], 0).sum())]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 # ======================================================================================================
@@ -430,6 +458,10 @@ def run_own(args):
     kms = eng.kernel_ms(min(64, args.steps))
     clocks = sampler.stop() if sampler else None
     value = world * n * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:            # the buffers still hold the last timed step's lists (batch (steps - 1) % B)
+        m = int(d_needed.item())
+        assert m <= d_ids.numel(), "the last timed step's ids did not fit the output buffer"
+        _dump_outputs(args.dump_outputs, d_spans.cpu().numpy().view(np.uint32), d_ids[:m].cpu().numpy().view(np.uint32), d_status.cpu().numpy())
 
     # the same loop in descriptor mode (8 B per matched filter instead of 4 B per matched id): explains the e2e number
     d_desc = torch.empty((int(desc_max * 1.25) + 1024, 2), dtype=torch.int32, device=dev)

@@ -133,8 +133,8 @@ class _FakeLib:
         self.bufs = {}
         self._real = real
 
-    def __getattr__(self, name):                 # pure host functions (gm_shard_of ...) are the real library's
-        if name.startswith("gm") and self._real is not None:
+    def __getattr__(self, name):                 # pure host functions (gm_shard_of ...) are the real library's; the router's gmr_* are
+        if name.startswith("gm_") and self._real is not None:      # not served, also where a device would let them run
             return getattr(self._real, name)
         raise AttributeError(name)
 
@@ -210,7 +210,8 @@ def fake_gpu(monkeypatch):
 
 
 def _ns(**kw):
-    d = dict(gpus=1, steps=3, warmup=3, impl="own", subs=20_000, topics=2_000, batches=2, no_cpu_baseline=False, e2e_steps=None, no_c4=False)
+    d = dict(gpus=1, steps=3, warmup=3, impl="own", subs=20_000, topics=2_000, batches=2, no_cpu_baseline=False, e2e_steps=None, no_c4=False,
+             dump_outputs=None)
     d.update(kw)
     return argparse.Namespace(**d)
 
@@ -307,6 +308,49 @@ def test_abnormal_ends_print_the_partial_line_once(mode, env, rc, printed, tmp_p
     if printed:
         d = json.loads(lines[0])
         assert d["value"] == 1.5 and "bench" in d["errors"]
+
+
+@pytest.mark.parametrize("steps, batch", [(2, 1), (3, 0)])
+def test_dump_outputs_holds_the_lists_of_the_last_timed_step(fake_gpu, tmp_path, steps, batch):
+    """--dump-outputs: the sorted per-topic lists of the batch the last timed step matched (step k matches batch k % batches),
+    as float64, equal to the oracle's lists of that batch."""
+    from oracle import oracle as orc
+    from rmqtt_b200 import workload as wl
+    bench, out = fake_gpu
+    args = _ns(steps=steps, batches=2, no_cpu_baseline=True, dump_outputs=str(tmp_path / "dump"))
+    bench.run_own(args)
+    d = {k: np.load(tmp_path / "dump" / f"{k}.npy") for k in ("topics", "status", "counts", "ids")}
+    assert all(a.dtype == np.float64 for a in d.values())
+    cfg = bench._cfg(args)
+    tree = orc.TopicTree()
+    tree.bulk_insert(*wl.gen_subs(cfg))
+    want = tree.match_batch(*wl.gen_topics(cfg, cfg.n_topics, stream=batch))
+    seg = np.repeat(np.arange(cfg.n_topics), np.maximum(want["counts"], 0))
+    assert (d["topics"] == np.arange(cfg.n_topics)).all() and (d["status"] == 0).all()
+    assert (d["counts"] == want["counts"]).all() and (d["ids"] == want["ids"][np.lexsort((want["ids"], seg))]).all()
+
+
+def test_dump_outputs_samples_a_large_batch_the_same_way_within_the_byte_budget(tmp_path, monkeypatch):
+    import bench
+    from rmqtt_b200.engine import MatchResult
+    n, per = 5000, 7
+    spans = np.stack([np.arange(n, dtype=np.uint32) * per, np.full(n, per, np.uint32)], axis=1)
+    ids = np.random.default_rng(1).integers(0, 1 << 32, n * per, dtype=np.uint64).astype(np.uint32)
+    status = np.zeros(n, np.int32)
+    status[::97] = -2
+    monkeypatch.setattr(bench, "_DUMP_TOPICS", 1000)
+    monkeypatch.setattr(bench, "_DUMP_BYTES", 8 * 6000)      # about 600 of the 1000 sampled topics fit (topic, status, count, 7 ids)
+    for run in ("a", "b"):
+        bench._dump_outputs(str(tmp_path / run), spans, ids, status)
+    d = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in ("topics", "status", "counts", "ids")}
+    for k, a in d.items():
+        assert (a == np.load(tmp_path / "b" / f"{k}.npy")).all(), k
+    t = d["topics"].astype(np.int64)
+    assert 600 <= len(t) < 1000 and (np.diff(t) > 0).all() and t[-1] > len(t)
+    counts, sorted_ids = MatchResult(spans[t], ids, status[t], len(ids)).canonical()
+    assert (d["status"] == status[t]).all() and (d["counts"] == counts).all() and (d["ids"] == sorted_ids).all()
+    words = sum(a.size for a in d.values())
+    assert 6000 - (3 + per) < words <= 6000                 # the next sampled topic would not have fit
 
 
 def test_a_missed_gather_barrier_keeps_the_fused_timings(fake_gpu, monkeypatch):
