@@ -25,6 +25,7 @@
 #include "relations.cuh"
 #include "retain_kernels.cuh"
 #include "retain_tree.h"
+#include "pipeline.h"
 #include "router_host.h"
 
 using namespace gm;
@@ -68,20 +69,30 @@ struct DevBuf {   // owning device allocation (freed on destruction, also on the
     template <class T> T* as() const { return static_cast<T*>(p); }
 };
 
-struct Ctrl {                       // device control block, zeroed before every match
-    unsigned long long cursor;
-    unsigned long long stats[24];
-    u32 slow_count;
-    u32 tile_counter;
-};
-
 static_assert(GM_ERR_INVALID_TOPIC == -2, "k_tokenize writes the per-topic status code directly");
 
-// fast-path geometry (see DESIGN.md): one topic per thread, 512 threads per CTA, 3 CTAs per SM (64 KB of shared memory each)
-constexpr int K2_FAST_L = 8;       // levels staged in shared memory; deeper topics take the deferred kernel
-constexpr int K2_THREADS = 512;
-constexpr int K2_CTAS_PER_SM = 3;
-constexpr u32 K2_POOL_ROWS = 24;   // matched value sets per topic beyond the 8 held in shared memory, before the topic is deferred
+// pipeline.h's launcher on a CUDA stream: counts the launches in *launches; the timing points go to one slot of the event ring
+struct CudaLauncher {
+    cudaStream_t s;
+    cudaEvent_t* ev;                // the ring slot, or nullptr: no timing
+    u64* ring_n;
+    u64* launches;
+    template <class... P, class... A>
+    int launch(void (*k)(P...), u32 grid, u32 block, size_t smem, A... a) {
+        k<<<grid, block, smem, s>>>(a...);
+        ++*launches;
+        CUDA_TRY(cudaGetLastError());
+        return GM_OK;
+    }
+    int memset(void* p, int v, size_t bytes) { CUDA_TRY(cudaMemsetAsync(p, v, bytes, s)); return GM_OK; }
+    int copy(void* dst, const void* src, size_t bytes) { CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); return GM_OK; }
+    int mark(int i) {
+        if (!ev) return GM_OK;
+        CUDA_TRY(cudaEventRecord(ev[i], s));
+        if (i == 3) ++*ring_n;
+        return GM_OK;
+    }
+};
 
 }  // namespace
 
@@ -147,8 +158,7 @@ struct gm_engine {
     u64 view_epoch = 0;               // bumped by every flush that changed what the kernels see
     // device tables
     DevBuf d_edges, d_ranges, d_values, d_dict, d_pool, d_cfilter, d_tree_slots;
-    size_t up_ranges = 0, up_values = 0, up_pool = 0, up_edges_slots = 0, up_dict_slots = 0;
-    u64 up_values_epoch = 0;
+    ShipMarks up;                    // what the device tables hold
     // flush staging: patches are gathered into PINNED host memory and scattered by kernels on the side stream —
     // the flush never synchronises the host with the device
     DevBuf d_patch;
@@ -165,12 +175,9 @@ struct gm_engine {
     u64 launches = 0;
     bool k2_attr_set = false;
     // fused gather over peer memory (comm.cuh): one block per rank holding every rank's slab; the peers' blocks are opened by CUDA IPC
-    struct Gather {
-        char* block = nullptr; size_t bytes = 0;
-        u32 world = 0, rank = 0, epoch = 0;
-        u64 slab_topics = 0, slab_ids = 0;
-        static constexpr size_t off_ids = 256;      // the block starts with a 256-byte header {world, slab_topics, slab_ids}
-        size_t off_spans = 0, off_index = 0, off_counts = 0, off_flags = 0;
+    struct Gather : GatherLayout {
+        char* block = nullptr;
+        u32 rank = 0, epoch = 0;
         char* peer[8] = {};
         DevBuf d_ptrs;      // device arrays for k_gather_finish: counts pointers [8], flags pointers [8]
         bool connected = false;
@@ -201,20 +208,6 @@ struct gm_engine {
     // GM_FLAG_MANUAL_FLUSH the host mirror may already have grown / re-hashed a table that the device has not seen yet.
     TrieView dev_view{};
     RetainView dev_rview{};
-    size_t up_rkids = 0, up_rvals = 0, up_redges_slots = 0;
-    TrieView view() const {
-        TrieView v{};
-        v.edges = d_edges.as<EdgeSlot>(); v.ranges = d_ranges.as<Range>();
-        v.values = d_values.as<u32>(); v.dict = d_dict.as<DictSlot>(); v.pool = d_pool.as<u8>();
-        v.cfilter = d_cfilter.as<u32>(); v.cfilter_mask = static_cast<u32>(trie.cfilter.size() - 1);
-        v.edge_mask = static_cast<u32>(trie.edges.size() - 1);
-        v.win_mask = trie.win_mask(); v.win_shift = trie.win_shift(); v.nwin_mask = trie.nwin_mask();
-        v.dict_mask = static_cast<u32>(trie.dict.size() - 1);
-        v.root_plus = trie.root_plus; v.root_hash_ref = trie.root_hash_ref; v.root_hash_cnt = trie.root_hash_cnt; v.root_mask = trie.root_mask;
-        v.max_depth = trie.max_depth;
-        v.tree_slots = d_tree_slots.as<u32>(); v.n_trees = d_tree_slots.p ? static_cast<u32>(trie.tree_slots.size()) : 0u;
-        return v;
-    }
 
     // ---- flush: ship the staged mutations to HBM on the side stream WITHOUT stopping the matches ------------------------
     // Phase A (no fence; only the host-mirror lock `mu` is held, matches keep running):
@@ -237,6 +230,14 @@ struct gm_engine {
     char* h_arena_[2] = {nullptr, nullptr}; size_t h_arena_cap_[2] = {0, 0};
     cudaEvent_t ev_arena_[2] = {nullptr, nullptr}; bool arena_pending_[2] = {false, false};
 
+    MatchGeometry geometry() const {
+        MatchGeometry g;
+        g.num_sms = static_cast<u32>(num_sms); g.k2_ctas = knobs.k2_ctas; g.site_bits = knobs.site_bits; g.sub_bits = knobs.sub_bits;
+        g.sorted_rows = knobs.sorted_rows; g.tok_bulk = knobs.tok_bulk; g.gather_direct = knobs.gather_direct;
+        g.diag_flags = knobs.diag_flags; g.tile_chunk = knobs.tile_chunk;
+        return g;
+    }
+
     int stage_reserve(size_t bytes) {
         if (bytes <= h_arena_cap_[arena_]) return GM_OK;
         size_t ncap = std::max(bytes, h_arena_cap_[arena_] * 2 + (size_t(1) << 20));
@@ -247,9 +248,10 @@ struct gm_engine {
         return GM_OK;
     }
 
+    // ---- the shipper of pipeline.h's ship() ----
     // gather the listed (already final) host slots into the pinned arena; they are scattered in phase B
     template <class V>
-    int stage_patches(DevBuf& buf, const V& host, std::vector<u32>& dirty) {
+    int patch(DevBuf& buf, const V& host, std::vector<u32>& dirty) {
         using T = std::remove_cv_t<std::remove_reference_t<decltype(host[0])>>;
         static_assert(sizeof(T) == 32 || sizeof(T) == 8 || sizeof(T) == 4 || sizeof(T) == 1, "patchable element sizes");
         std::sort(dirty.begin(), dirty.end());
@@ -271,65 +273,20 @@ struct gm_engine {
     }
 
     // whole array into a fresh device buffer (swapped in at the fence)
-    template <class V>
-    int stage_fresh(DevBuf& buf, const V& host, size_t min_bytes, size_t slack_bytes = 0) {
-        using T = std::remove_cv_t<std::remove_reference_t<decltype(host[0])>>;
-        DevBuf fresh;
-        CUDA_TRY(fresh.ensure(std::max<size_t>(std::max(host.size() * sizeof(T) + slack_bytes, min_bytes), 256)));
-        if (host.size()) CUDA_TRY(cudaMemcpyAsync(fresh.p, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice, side));
-        swaps_.push_back(Swap{&buf, std::move(fresh)});
+    int fresh(DevBuf& buf, const void* src, size_t bytes, size_t cap_bytes) {
+        DevBuf nb;
+        CUDA_TRY(nb.ensure(cap_bytes));
+        if (bytes) CUDA_TRY(cudaMemcpyAsync(nb.p, src, bytes, cudaMemcpyHostToDevice, side));
+        swaps_.push_back(Swap{&buf, std::move(nb)});
         return GM_OK;
     }
-
-    // Hash tables (edges, dict): whole table into a new buffer after a re-hash or when most of it changed, else patches.
-    template <class V>
-    int upload_table(DevBuf& buf, const V& host, bool& full, std::vector<u32>& dirty, size_t& up_slots) {
-        int st;
-        if (full || up_slots != host.size() || dirty.size() * 8 > host.size()) {
-            if ((st = stage_fresh(buf, host, 0)) != GM_OK) return st;
-            up_slots = host.size();
-            dirty.clear();
-        } else if ((st = stage_patches(buf, host, dirty)) != GM_OK) return st;
-        full = false;
+    // a tail behind the part the running kernels can reach
+    int append(DevBuf& buf, size_t off, const void* src, size_t bytes) {
+        CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(buf.p) + off, src, bytes, cudaMemcpyHostToDevice, side));
         return GM_OK;
     }
-
-    // Append-only arrays (ranges, values, pool, retained child blocks / values): copy the new tail in place (no running
-    // kernel can reach it yet); a grown or rebuilt array goes into a new buffer; older entries that changed are patched.
-    template <class V>
-    int upload_appendable(DevBuf& buf, const V& host, size_t& up, std::vector<u32>* dirty) {
-        using T = std::remove_cv_t<std::remove_reference_t<decltype(host[0])>>;
-        const size_t bytes = host.size() * sizeof(T);
-        if ((up == 0 && (host.size() > 0 || !buf.p)) || bytes > buf.cap) {    // first shipment, rebuilt content, or out of room: new buffer with room to append
-            int st = stage_fresh(buf, host, std::max(bytes * 2, size_t(4096)));
-            if (st != GM_OK) return st;
-            up = host.size();
-            if (dirty) dirty->clear();
-            return GM_OK;
-        }
-        const size_t before = up;
-        if (host.size() > up) {
-            CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(buf.p) + up * sizeof(T), host.data() + up, (host.size() - up) * sizeof(T), cudaMemcpyHostToDevice, side));
-            up = host.size();
-        }
-        if (dirty) {
-            dirty->erase(std::remove_if(dirty->begin(), dirty->end(), [&](u32 i) { return i >= before; }), dirty->end());
-            int st = stage_patches(buf, host, *dirty);
-            if (st != GM_OK) return st;
-            dirty->clear();
-        }
-        return GM_OK;
-    }
-
-    RetainView rview() const {
-        RetainView v{};
-        v.kids = d_rkids.as<RKid>(); v.edges = d_redges.as<REdge>(); v.vals = d_rvals.as<u32>();
-        v.edge_mask = static_cast<u32>(rtree.redges.size() - 1);
-        if (!rtree.rnodes.empty()) { v.root_first_kid = rtree.rnodes[0].first_kid; v.root_nk_flags = rtree.rnodes[0].nkids | (rtree.rnodes[0].flags << 28); }
-        v.root_plain_kids = rtree.root_plain_kids; v.root_plain_val_hi = rtree.root_plain_val_hi; v.max_depth = rtree.max_depth;
-        v.n_kids = static_cast<u32>(rtree.rkids.size());
-        return v;
-    }
+    size_t capacity(const DevBuf& buf) const { return buf.cap; }
+    TableBufs<DevBuf> tables() { return {&d_edges, &d_dict, &d_ranges, &d_values, &d_pool, &d_cfilter, &d_tree_slots, &d_rnodes, &d_rkids, &d_redges, &d_rvals}; }
 
     void free_retired(bool all) {
         if (retired.empty()) return;
@@ -345,9 +302,8 @@ struct gm_engine {
         const int st = flush_impl();
         if (st != GM_OK && !(flags & GM_FLAG_HOST_ONLY) && st != GM_ERR_TOO_LARGE) {
             jobs_.clear(); swaps_.clear(); stage_used_ = 0;               // (fresh buffers not yet swapped in are freed here)
-            up_ranges = up_values = up_pool = 0; up_edges_slots = up_dict_slots = 0;
+            up.forget_all();
             trie.full_edges = trie.full_dict = true; trie.cfilter_dirty = true; trie.trees_dirty = true; trie.root_dirty = true;
-            up_rkids = up_rvals = up_redges_slots = 0;
             rtree.dirty = true; rtree.full = true;
         }
         return st;
@@ -362,45 +318,14 @@ struct gm_engine {
         if (!trie.any_dirty() && !rtree.dirty) return GM_OK;
         CUDA_TRY(cudaSetDevice(device));
         if (!trie.sync()) { g_err = "more than 2^32 live value words"; return GM_ERR_TOO_LARGE; }
-        if (trie.values_epoch != up_values_epoch) { up_values = up_ranges = 0; up_values_epoch = trie.values_epoch; }   // value sets were compacted: re-ship whole
         free_retired(false);
         // ---------------- phase A ----------------
         arena_ ^= 1;
         if (arena_pending_[arena_]) { CUDA_TRY(cudaEventSynchronize(ev_arena_[arena_])); arena_pending_[arena_] = false; }   // two flushes ago: long done
         jobs_.clear(); swaps_.clear(); stage_used_ = 0;
-        int rs;
         bool r_shipped = false;
-        if (rtree.dirty) {   // retained tree: whole arrays after a (re)flatten, else only the entries set / remove edited in place
-            rtree.prepare_flush();
-            if (rtree.full) {
-                const std::vector<u32> marker{0u};       // "retained tree shipped" (records travel in rkids / redges)
-                if ((rs = stage_fresh(d_rnodes, marker, 0)) != GM_OK) return rs;
-                if ((rs = stage_fresh(d_rkids, rtree.rkids, 0, (rtree.rkids.size() / 4 + 1024) * sizeof(RKid))) != GM_OK) return rs;   // room for in-place appends
-                if ((rs = stage_fresh(d_redges, rtree.redges, 0)) != GM_OK) return rs;
-                if ((rs = stage_fresh(d_rvals, rtree.rvals, 0, 4096)) != GM_OK) return rs;
-                up_rkids = rtree.rkids.size(); up_rvals = rtree.rvals.size(); up_redges_slots = rtree.redges.size();
-            } else {
-                bool full_edges = false;
-                if ((rs = upload_appendable(d_rkids, rtree.rkids, up_rkids, &rtree.dirty_kids)) != GM_OK) return rs;
-                if ((rs = upload_table(d_redges, rtree.redges, full_edges, rtree.dirty_edges, up_redges_slots)) != GM_OK) return rs;
-                if ((rs = upload_appendable(d_rvals, rtree.rvals, up_rvals, &rtree.dirty_vals)) != GM_OK) return rs;
-            }
-            r_shipped = true;
-        }
-        if ((rs = upload_table(d_edges, trie.edges, trie.full_edges, trie.dirty_edges, up_edges_slots)) != GM_OK) return rs;
-        if ((rs = upload_table(d_dict, trie.dict, trie.full_dict, trie.dirty_dict, up_dict_slots)) != GM_OK) return rs;
-        if ((rs = upload_appendable(d_ranges, trie.ranges, up_ranges, nullptr)) != GM_OK) return rs;
-        if ((rs = upload_appendable(d_values, trie.values, up_values, nullptr)) != GM_OK) return rs;
-        if ((rs = upload_appendable(d_pool, trie.pool, up_pool, nullptr)) != GM_OK) return rs;
-        if (trie.cfilter_dirty) {   // child filter of wide nodes: a few MB, shipped whole into a new buffer (a rebuild changes its geometry)
-            if ((rs = stage_fresh(d_cfilter, trie.cfilter, 0)) != GM_OK) return rs;
-            trie.cfilter_dirty = false;
-        }
-        if (trie.trees_dirty) {      // root records of the extra trees (ACL rules, rewrite rules, ...): a tiny array, shipped whole
-            if ((rs = stage_fresh(d_tree_slots, trie.tree_slots, 0)) != GM_OK) return rs;
-            trie.trees_dirty = false;
-        }
-        trie.root_dirty = false;
+        const int rs = ship(*this, tables(), trie, rtree, up, &r_shipped);
+        if (rs != GM_OK) return rs;
         if (stage_used_) {
             CUDA_TRY(d_patch.ensure(stage_used_));
             CUDA_TRY(cudaMemcpyAsync(d_patch.p, h_arena_[arena_], stage_used_, cudaMemcpyHostToDevice, side));
@@ -426,8 +351,9 @@ struct gm_engine {
             }
             CUDA_TRY(cudaGetLastError());
             if (stage_used_) { CUDA_TRY(cudaEventRecord(ev_arena_[arena_], side)); arena_pending_[arena_] = true; }
-            dev_view = view();
-            dev_rview = rview();
+            dev_view = make_trie_view(trie, {d_edges.as<EdgeSlot>(), d_ranges.as<Range>(), d_values.as<u32>(), d_dict.as<DictSlot>(), d_pool.as<u8>(),
+                                             d_cfilter.as<u32>(), d_tree_slots.as<u32>()});
+            dev_rview = make_retain_view(rtree, {d_rkids.as<RKid>(), d_redges.as<REdge>(), d_rvals.as<u32>()});
             view_epoch++;
             CUDA_TRY(cudaEventRecord(ev_flush, side));
             flush_gen++;
@@ -438,180 +364,68 @@ struct gm_engine {
 
     std::vector<MatchCtx*> all_ctxs() { std::vector<MatchCtx*> v; for (auto& c : ctxs) v.push_back(&c); v.push_back(&devctx); return v; }
 
-    // ---- the match pipeline, all on `s`, all buffers on the device; scratch from context `c` (caller holds mu_dev) ----
-    // `desc`: descriptor mode (d_ids_ is then a uint2 array of value-set references, cap_ids counts descriptors).
-    // `d_sel`: optional selection — row t matches entry d_sel[t] of the packed batch (n = number of selected rows).
-    // `hdr` (small-batch graphs only): device words {n, blob_bytes} read by the kernels at run time; n is then the CAPACITY.
-    int enqueue_match(MatchCtx& c, const void* d_blob_, u64 blob_bytes, const u32* d_offs_, u64 n, gm_span* d_spans_, void* d_ids_, u64 cap_ids,
-                      u64* d_needed, int32_t* d_status_, cudaStream_t s, bool stats, bool keep_cursor = false, bool desc = false,
-                      const u32* d_sel = nullptr, u64 readable_bytes = 0, const u32* hdr = nullptr, bool timing = true, u32 site_bits_override = 0,
-                      const u32* d_trees = nullptr, bool gather_mode = false) {
-        if (n == 0) { if (d_needed) CUDA_TRY(cudaMemsetAsync(d_needed, 0, sizeof(u64), s)); return GM_OK; }
-        if (n > 0xFFFFFFF0ull) { g_err = "batch too large"; return GM_ERR_TOO_LARGE; }
-        if (cap_ids > 0xFFFFFFFFull) cap_ids = 0xFFFFFFFFull;   // spans carry 32-bit offsets
-        const u32 n32 = static_cast<u32>(n);
-        const u32 S = std::max<u32>(1u, dev_view.max_depth);
-        CUDA_TRY(c.d_tok.ensure(S > TOK8 ? static_cast<size_t>(S) * n32 * sizeof(u32) : 256));
-        CUDA_TRY(c.d_tok8.ensure(static_cast<size_t>(n32) * TOK8 * sizeof(u32)));
-        CUDA_TRY(c.d_meta.ensure(n32 * sizeof(u32)));
-        CUDA_TRY(c.d_slow.ensure(n32 * sizeof(u32)));
-        CUDA_TRY(c.d_ctrl.ensure(sizeof(Ctrl)));
-        // locality pass scratch: bkey[n], perm[n]; hist + cursor [NBUCKETS] each
-        CUDA_TRY(c.d_sort.ensure(static_cast<size_t>(n32) * 11 * sizeof(u32) + 64));
-        const u32 site_bits = site_bits_override ? site_bits_override : knobs.site_bits, sub_bits = site_bits_override ? 0u : knobs.sub_bits;
-        const u32 NBUCKETS = 1u << (site_bits + sub_bits);
-        CUDA_TRY(c.d_hist.ensure(2 * static_cast<size_t>(NBUCKETS) * sizeof(u32)));
-        u32* bkey = c.d_sort.as<u32>();
-        u32* perm = bkey + n32;
-        u32* meta_sorted = perm + n32;
-        u32* tok8_sorted = meta_sorted + n32 + ((8 - (3 * static_cast<size_t>(n32)) % 8) % 8);   // 32-byte aligned rows
-        const bool sorted_rows = knobs.sorted_rows;
-        u32* hist = c.d_hist.as<u32>();
-        u32* bcursor = hist + NBUCKETS;
-        const bool small = hdr != nullptr;
-        const int k3_blocks = small ? std::max(1, std::min<int>(num_sms, (n32 + 7) / 8)) : num_sms * 4;
-        const u32 stack_cap = 32u * (dev_view.max_depth + 2u) + 64u;
-        CUDA_TRY(c.d_gstack.ensure(static_cast<size_t>(num_sms) * 4 * 8 * stack_cap * sizeof(u64)));
-        const int k2_ctas = (knobs.k2_ctas >= 1 && knobs.k2_ctas <= K2_CTAS_PER_SM) ? knobs.k2_ctas : K2_CTAS_PER_SM;
-        const int k2_grid = small ? std::max(1, std::min<int>(num_sms * k2_ctas, (n32 + K2_THREADS - 1) / K2_THREADS)) : num_sms * k2_ctas;
-        CUDA_TRY(c.d_gpool.ensure(static_cast<size_t>(num_sms) * k2_ctas * K2_THREADS * K2_POOL_ROWS * sizeof(Desc)));
+    // ---- the match pipeline (pipeline.h), all on `s`, all buffers on the device; scratch from context `c` (caller holds mu_dev) ----
+    int enqueue_match(MatchCtx& c, const MatchJob& j, cudaStream_t s) {
+        if (j.n == 0) { if (j.d_needed) CUDA_TRY(cudaMemsetAsync(j.d_needed, 0, sizeof(u64), s)); return GM_OK; }
+        if (j.n > 0xFFFFFFF0ull) { g_err = "batch too large"; return GM_ERR_TOO_LARGE; }
+        const MatchGeometry g = geometry();
+        const MatchPlan p = plan_match(g, j, dev_view.max_depth);
+        CUDA_TRY(c.d_tok.ensure(p.tok));
+        CUDA_TRY(c.d_tok8.ensure(p.tok8));
+        CUDA_TRY(c.d_meta.ensure(p.meta));
+        CUDA_TRY(c.d_slow.ensure(p.slow));
+        CUDA_TRY(c.d_ctrl.ensure(p.ctrl));
+        CUDA_TRY(c.d_sort.ensure(p.sort));
+        CUDA_TRY(c.d_hist.ensure(p.hist));
+        CUDA_TRY(c.d_gstack.ensure(p.gstack));
+        CUDA_TRY(c.d_gpool.ensure(p.gpool));
+        const bool small = j.hdr != nullptr;
         if (!small) {      // (a captured graph carries these dependencies as its launch order; events of other streams cannot be waited on while capturing)
             CUDA_TRY(cudaStreamWaitEvent(s, ev_flush, 0));
             if (c.recorded) CUDA_TRY(cudaStreamWaitEvent(s, c.ev_done, 0));   // this context's scratch: one match at a time
         }
-        // the bump cursor over out_ids survives between the chunks of one pipelined host call
-        if (keep_cursor) CUDA_TRY(cudaMemsetAsync(static_cast<char*>(c.d_ctrl.p) + sizeof(unsigned long long), 0, sizeof(Ctrl) - sizeof(unsigned long long), s));
-        else CUDA_TRY(cudaMemsetAsync(c.d_ctrl.p, 0, sizeof(Ctrl), s));
-        CUDA_TRY(cudaMemsetAsync(hist, 0, NBUCKETS * sizeof(u32), s));
-        Ctrl* ctrl = c.d_ctrl.as<Ctrl>();
-        const TrieView tv = dev_view;
-
-        cudaEvent_t* ev_t = ev_ring[ring_n % RING];
-        if (timing) CUDA_TRY(cudaEventRecord(ev_t[0], s));
-        auto k1 = knobs.tok_bulk ? k_tokenize<true> : k_tokenize<false>;
-        k1<<<(n32 + TOK_THREADS - 1) / TOK_THREADS, TOK_THREADS, 0, s>>>(
-            static_cast<const u8*>(d_blob_), static_cast<u32>(blob_bytes), static_cast<u32>(std::max<u64>(blob_bytes, readable_bytes)), d_offs_, d_sel, n32, hdr, tv, S,
-            c.d_tok8.as<u32>(), c.d_tok.as<u32>(), c.d_meta.as<u32>(), d_status_, bkey, hist, site_bits, sub_bits);
-        k_bucket_scan<<<1, 1024, 0, s>>>(hist, bcursor, NBUCKETS);
-        k_bucket_scatter<<<(n32 + 255) / 256, 256, 0, s>>>(bkey, bcursor, n32, hdr, perm, c.d_tok8.as<u32>(), c.d_meta.as<u32>(),
-                                                            sorted_rows ? tok8_sorted : nullptr, meta_sorted);
-        CUDA_TRY(cudaGetLastError());
-        if (timing) CUDA_TRY(cudaEventRecord(ev_t[1], s));
-
-        MatchParams mp{};
-        mp.tv = tv; mp.tok8 = c.d_tok8.as<u32>(); mp.tok = c.d_tok.as<u32>(); mp.meta = c.d_meta.as<u32>(); mp.n = n32; mp.n_ptr = hdr; mp.tok_levels = S;
-        mp.spans = reinterpret_cast<uint2*>(d_spans_); mp.out_ids = static_cast<u32*>(d_ids_); mp.out_desc = static_cast<uint2*>(d_ids_); mp.cap_ids = cap_ids;
-        mp.status = d_status_;
-        mp.trees = d_trees;
-        mp.cursor = &ctrl->cursor; mp.slow_list = c.d_slow.as<u32>(); mp.slow_count = &ctrl->slow_count;
-        mp.tile_counter = &ctrl->tile_counter; mp.stats = ctrl->stats;
-        mp.perm = perm; mp.tok8_sorted = tok8_sorted; mp.meta_sorted = meta_sorted;
-        mp.flags = (sorted_rows ? MP_SORTED_ROWS : 0u) | knobs.diag_flags;
-        mp.tile_chunk = knobs.tile_chunk;
-        if (gather_mode) {
-            const Gather& g = gather;
-            mp.g_base_topics = static_cast<u32>(g.rank * g.slab_topics); mp.g_base_ids = g.rank * g.slab_ids; mp.g_sel = d_sel;
-            if (knobs.gather_direct) {          // the publish phase stores into every rank's block itself
-                mp.g_world = g.world;
-                for (u32 w = 0; w < g.world; ++w) {
-                    mp.g_ids[w] = reinterpret_cast<u32*>(g.peer[w] + Gather::off_ids); mp.g_spans[w] = reinterpret_cast<uint2*>(g.peer[w] + g.off_spans);
-                    mp.g_index[w] = reinterpret_cast<u32*>(g.peer[w] + g.off_index);
-                }
-            } else {                            // ... into its own block only; k_gather_push copies the slab to the peers
-                mp.g_world = 1;
-                mp.g_ids[0] = reinterpret_cast<u32*>(g.block + Gather::off_ids); mp.g_spans[0] = reinterpret_cast<uint2*>(g.block + g.off_spans);
-                mp.g_index[0] = reinterpret_cast<u32*>(g.block + g.off_index);
-            }
-        }
-        constexpr size_t k2_smem = k2_smem_bytes<K2_FAST_L, K2_THREADS>();
-        auto k2_ss = k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, true, false>;
-        auto k2_sd = k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, true, true>;
-        auto k2_ns = k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, false>;
-        auto k2_nd = k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, true>;
-        auto k2_g = k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, false, true>;
         if (!k2_attr_set) {
-            for (auto k : {k2_ss, k2_sd, k2_ns, k2_nd, k2_g}) CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(k2_smem)));
+            for (MatchFastKernel k : match_fast_kernels())
+                CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(k2_smem_bytes<K2_FAST_L, K2_THREADS>())));
             k2_attr_set = true;
         }
-        (gather_mode ? k2_g : stats ? (desc ? k2_sd : k2_ss) : (desc ? k2_nd : k2_ns))<<<k2_grid, K2_THREADS, k2_smem, s>>>(mp, c.d_gpool.as<Desc>(), K2_POOL_ROWS);
-        CUDA_TRY(cudaGetLastError());
-        if (timing) CUDA_TRY(cudaEventRecord(ev_t[2], s));
-        auto k3 = gather_mode ? k_match_slow<false, false, true>
-                              : stats ? (desc ? k_match_slow<true, true> : k_match_slow<true, false>) : (desc ? k_match_slow<false, true> : k_match_slow<false, false>);
-        k3<<<k3_blocks, 256, 0, s>>>(mp, c.d_gstack.as<u64>(), stack_cap);
-        CUDA_TRY(cudaGetLastError());
-        if (timing) { CUDA_TRY(cudaEventRecord(ev_t[3], s)); ring_n++; }
-        launches += 5;
-        if (d_needed) CUDA_TRY(cudaMemcpyAsync(d_needed, &ctrl->cursor, sizeof(u64), cudaMemcpyDeviceToDevice, s));
+        CudaLauncher l{s, j.timing ? ev_ring[ring_n % RING] : nullptr, &ring_n, &launches};
+        const int st = match_pipeline(l, g, j, p, dev_view, {c.d_tok.as<u32>(), c.d_tok8.as<u32>(), c.d_meta.as<u32>(), c.d_slow.as<u32>(), c.d_ctrl.as<Ctrl>(),
+                                                          c.d_sort.as<u32>(), c.d_hist.as<u32>(), c.d_gstack.as<u64>(), c.d_gpool.as<Desc>()});
+        if (st != GM_OK) return st;
         if (!small) { CUDA_TRY(cudaEventRecord(c.ev_done, s)); c.recorded = true; }
         return GM_OK;
     }
 
-    // ---- retained lookup: tokenise filters -> frontier BFS (one step kernel per tree level) -> publish ----
-    struct RCtl { unsigned long long grand; unsigned long long stats[2]; u32 err; u32 pad; u32 n_desc[RQ]; u32 counts[RQ]; };   // counts[(max_depth + 3) * RQ], then claim[max_depth + 3] follow   // counts[(max_depth + 3) * RQ] follow
-
-    int enqueue_retain(const void* d_blob_, u64 blob_bytes, const u32* d_offs_, u64 n, gm_span* d_spans_, u32* d_ids_, u64 cap_ids, int32_t* d_status_, cudaStream_t s) {
+    // ---- retained lookup (pipeline.h) on the engine-wide scratch ----
+    int enqueue_retain(const RetainJob& j, cudaStream_t s) {
         std::lock_guard<std::mutex> gd(mu_dev);     // enqueue only; the caller (holding mu_ret) synchronises afterwards without it
         MatchCtx& c = devctx;
-        const u32 nq = static_cast<u32>(n);
-        const u32 depth = dev_rview.max_depth;
-        const u32 S = depth + 2;                       // the walk reads filter levels pos and pos+1 with pos <= tree depth
-        const size_t ctl_bytes = sizeof(RCtl) + static_cast<size_t>(depth + 3) * RQ * sizeof(u32) + static_cast<size_t>(depth + 3) * sizeof(u32);
-        CUDA_TRY(c.d_tok.ensure(S > TOK8 ? static_cast<size_t>(S) * nq * sizeof(u32) : 256));
-        CUDA_TRY(c.d_tok8.ensure(static_cast<size_t>(nq) * TOK8 * sizeof(u32)));
-        CUDA_TRY(c.d_meta.ensure(nq * sizeof(u32)));
-        CUDA_TRY(d_rq.ensure(static_cast<size_t>(nq) * 3 * sizeof(u32)));
-        CUDA_TRY(d_rctl.ensure(ctl_bytes));
-        const u32 slice_items = r_cap_items / RQ, slice_desc = r_cap_desc / RQ;   // queues are split into RQ slices
-        CUDA_TRY(d_rfront[0].ensure(static_cast<size_t>(slice_items) * RQ * sizeof(RTask)));
-        CUDA_TRY(d_rfront[1].ensure(static_cast<size_t>(slice_items) * RQ * sizeof(RTask)));
-        CUDA_TRY(d_rdescs.ensure(static_cast<size_t>(slice_desc) * RQ * sizeof(RDesc)));
+        const RetainPlan p = plan_retain(j.n, dev_rview.max_depth, r_cap_items, r_cap_desc);
+        CUDA_TRY(c.d_tok.ensure(p.tok));
+        CUDA_TRY(c.d_tok8.ensure(p.tok8));
+        CUDA_TRY(c.d_meta.ensure(p.meta));
+        CUDA_TRY(d_rq.ensure(p.rq));
+        CUDA_TRY(d_rctl.ensure(p.ctl));
+        CUDA_TRY(d_rfront[0].ensure(p.front));
+        CUDA_TRY(d_rfront[1].ensure(p.front));
+        CUDA_TRY(d_rdescs.ensure(p.descs));
         CUDA_TRY(cudaStreamWaitEvent(s, ev_flush, 0));
         if (c.recorded) CUDA_TRY(cudaStreamWaitEvent(s, c.ev_done, 0));
-        CUDA_TRY(cudaMemsetAsync(d_rctl.p, 0, ctl_bytes, s));
-        CUDA_TRY(cudaMemsetAsync(d_rq.p, 0, static_cast<size_t>(nq) * 3 * sizeof(u32), s));
-        RCtl* ctl = d_rctl.as<RCtl>();
-        u32* qtotal = d_rq.as<u32>();
-        u32* qbase = qtotal + nq;
-        u32* qcur = qbase + nq;
-        cudaEvent_t* ev_t = ev_ring[ring_n % RING];
-        CUDA_TRY(cudaEventRecord(ev_t[0], s));
-        k_tokenize<false><<<(nq + TOK_THREADS - 1) / TOK_THREADS, TOK_THREADS, 0, s>>>(static_cast<const u8*>(d_blob_), static_cast<u32>(blob_bytes), static_cast<u32>(blob_bytes), d_offs_, nullptr, nq, nullptr, dev_view, S, c.d_tok8.as<u32>(), c.d_tok.as<u32>(), c.d_meta.as<u32>(), d_status_, nullptr, nullptr, 0u, 0u);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaEventRecord(ev_t[1], s));
-        RetainParams rp{};
-        rp.v = dev_rview; rp.qtok8 = c.d_tok8.as<u32>(); rp.qtok = c.d_tok.as<u32>(); rp.qmeta = c.d_meta.as<u32>(); rp.nq = nq; rp.tok_levels = S;
-        rp.descs = d_rdescs.as<RDesc>(); rp.n_desc = ctl->n_desc; rp.cap_items = slice_items; rp.cap_desc = slice_desc;
-        rp.qtotal = qtotal; rp.err = &ctl->err;
-        // round 0 follows every filter's literal prefix; every later round expands the wildcard tasks the round before
-        // queued.  A task descends at least one tree level, so depth + 1 rounds drain every queue (late rounds find
-        // theirs empty and return at once).
-        rp.stats = ctl->stats;
-        auto kri = knobs.retain_stats ? k_retain_init<true> : k_retain_init<false>;
-        auto krr = knobs.retain_stats ? k_retain_round<true> : k_retain_round<false>;
-        kri<<<(nq + 255) / 256, 256, 0, s>>>(rp, d_rfront[0].as<RTask>(), &ctl->counts[0]);
-        const int grid = num_sms * 8;
-        const int rgrid = num_sms * GM_RETAIN_CTAS;   // exactly the resident CTAs (launch bound of k_retain_round): tasks are claimed dynamically
-        for (u32 lvl = 0; lvl <= depth; ++lvl)
-            krr<<<rgrid, 256, 0, s>>>(rp, d_rfront[lvl & 1].as<RTask>(), &ctl->counts[static_cast<size_t>(lvl) * RQ], d_rfront[(lvl + 1) & 1].as<RTask>(),
-                                      &ctl->counts[static_cast<size_t>(lvl + 1) * RQ], &ctl->counts[static_cast<size_t>(depth + 3) * RQ + lvl]);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaEventRecord(ev_t[2], s));
-        k_retain_scan<<<1, 1024, 0, s>>>(qtotal, nq, qbase, reinterpret_cast<uint2*>(d_spans_), &ctl->grand);
-        k_retain_expand<<<grid, 256, 0, s>>>(d_rdescs.as<RDesc>(), ctl->n_desc, slice_desc, dev_rview.vals, qbase, qcur, d_ids_, cap_ids);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaEventRecord(ev_t[3], s));
-        ring_n++;
-        launches += 4 + depth + 1;
+        CudaLauncher l{s, ev_ring[ring_n % RING], &ring_n, &launches};
+        const int st = retain_pipeline(l, j, p, dev_view, dev_rview, {c.d_tok.as<u32>(), c.d_tok8.as<u32>(), c.d_meta.as<u32>(), d_rq.as<u32>(), d_rctl.as<RCtl>(),
+                                                                   {d_rfront[0].as<RTask>(), d_rfront[1].as<RTask>()}, d_rdescs.as<RDesc>()}, static_cast<u32>(num_sms));
+        if (st != GM_OK) return st;
         CUDA_TRY(cudaEventRecord(c.ev_done, s));
         c.recorded = true;
         return GM_OK;
     }
 
     // runs the pipeline, growing the frontier / descriptor scratch until nothing overflowed; leaves *total
-    int run_retain(const void* d_blob_, u64 blob_bytes, const u32* d_offs_, u64 n, gm_span* d_spans_, u32* d_ids_, u64 cap_ids, int32_t* d_status_, cudaStream_t s, u64* total) {
-        for (int attempt = 0; attempt < 12; ++attempt) {
-            int st = enqueue_retain(d_blob_, blob_bytes, d_offs_, n, d_spans_, d_ids_, cap_ids, d_status_, s);
+    int run_retain(RetainJob j, cudaStream_t s, u64* total) {
+        j.stats = knobs.retain_stats;
+        for (int attempt = 0; attempt < RETAIN_ATTEMPTS; ++attempt) {
+            int st = enqueue_retain(j, s);
             if (st != GM_OK) return st;
             RCtl h{};
             CUDA_TRY(cudaMemcpyAsync(&h, d_rctl.p, sizeof(RCtl), cudaMemcpyDeviceToHost, s));
@@ -626,8 +440,7 @@ struct gm_engine {
                 fprintf(stderr, "; descriptors %llu\n", nd);
             }
             if (h.err == 0) { *total = h.grand; return GM_OK; }
-            if (h.err & 1u) { if (r_cap_items > (1u << 30)) break; r_cap_items *= 4; }
-            if (h.err & 2u) { if (r_cap_desc > (1u << 30)) break; r_cap_desc *= 4; }
+            if (!retain_grow(h.err, r_cap_items, r_cap_desc)) break;
         }
         g_err = "retained lookup: frontier does not fit the scratch limits, split the batch";
         return GM_ERR_TOO_LARGE;
@@ -784,9 +597,7 @@ int32_t gm_compact(gm_engine* e) {
     std::vector<u32> remap;
     e->trie.compact(&keep, &remap);
     e->rtree.remap_tokens(remap);
-    e->up_ranges = e->up_values = e->up_pool = 0;
-    e->up_values_epoch = e->trie.values_epoch;
-    e->up_edges_slots = e->up_dict_slots = 0;
+    e->up.forget_trie(e->trie.values_epoch);
     return (e->flags & GM_FLAG_HOST_ONLY) ? GM_OK : e->flush_locked();
 }
 
@@ -814,8 +625,12 @@ static int32_t match_device_impl(gm_engine* e, const void* d_blob, uint64_t blob
     { int st = auto_flush(e); if (st != GM_OK) return st; }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     std::unique_lock<std::mutex> gd(e->mu_dev);
-    int st = e->enqueue_match(e->devctx, d_blob, blob_bytes, d_offs, n, d_spans, d_out, cap, d_needed, d_status, s, work != nullptr, false, desc, d_sel, 0, nullptr, true, 0,
-                              d_trees);
+    MatchJob job;
+    job.blob = d_blob; job.blob_bytes = blob_bytes; job.offs = d_offs; job.sel = d_sel; job.n = n;
+    job.spans = d_spans; job.out = d_out; job.cap = cap; job.d_needed = d_needed; job.status = d_status; job.trees = d_trees;
+    job.mode = desc ? MatchJob::DESCRIPTORS : MatchJob::IDS;
+    job.stats = work != nullptr;
+    int st = e->enqueue_match(e->devctx, job, s);
     if (st != GM_OK || !work) return st;
     std::memset(work, 0, sizeof(*work));
     if (n == 0) return GM_OK;
@@ -909,9 +724,15 @@ static int small_graph_match(gm_engine* e, MatchCtx& c, std::unique_lock<std::mu
     auto enqueue = [&](cudaStream_t s) -> int {
         char* di = static_cast<char*>(g->d_in.p);
         char* dout = static_cast<char*>(g->d_out.p);
-        return e->enqueue_match(c, di + g->off_blob, g->cap_blob, reinterpret_cast<const u32*>(di + g->off_offs), g->cap_n, reinterpret_cast<gm_span*>(dout + g->off_spans),
-                                dout + g->off_out, g->cap_out, reinterpret_cast<u64*>(dout), reinterpret_cast<int32_t*>(dout + g->off_status), s, false, false, desc,
-                                nullptr, g->cap_blob, reinterpret_cast<const u32*>(di), false, 10u, reinterpret_cast<const u32*>(di + g->off_trees));
+        MatchJob j;
+        j.blob = di + g->off_blob; j.blob_bytes = j.readable_bytes = g->cap_blob; j.offs = reinterpret_cast<const u32*>(di + g->off_offs);
+        j.n = g->cap_n; j.hdr = reinterpret_cast<const u32*>(di);
+        j.spans = reinterpret_cast<gm_span*>(dout + g->off_spans); j.out = dout + g->off_out; j.cap = g->cap_out;
+        j.d_needed = reinterpret_cast<u64*>(dout); j.status = reinterpret_cast<int32_t*>(dout + g->off_status); j.trees = reinterpret_cast<const u32*>(di + g->off_trees);
+        j.mode = desc ? MatchJob::DESCRIPTORS : MatchJob::IDS;
+        j.timing = false;
+        j.bucket_bits = 10;
+        return e->enqueue_match(c, j, s);
     };
     if (!g->warmed) {      // allocate the scratch and set kernel attributes outside any capture: one empty (n = 0) pass
         CUDA_TRY(cudaMemsetAsync(g->d_in.p, 0, g->in_bytes, c.sc));
@@ -1032,9 +853,14 @@ static int32_t match_host_impl(gm_engine* e, const char* blob, const uint32_t* o
     for (int k = 0; k < nchunks; ++k) {
         const u64 c0 = k * chunk, c1 = std::min<u64>(n, c0 + chunk);
         CUDA_TRY(cudaStreamWaitEvent(c.sc, c.ev_h2d[k], 0));
-        int st = e->enqueue_match(c, c.d_blob.p, offsets[c1], c.d_offs.as<u32>() + c0, c1 - c0, c.d_spans.as<gm_span>() + c0, c.d_ids.p, cap_ids, nullptr,
-                                  c.d_status.as<int32_t>() + c0, c.sc, false, k != 0, desc, nullptr, (offsets[c1] + 15) & ~u64(15), nullptr, true, 0,
-                                  trees ? c.d_trees.as<u32>() + c0 : nullptr);
+        MatchJob j;
+        j.blob = c.d_blob.p; j.blob_bytes = offsets[c1]; j.readable_bytes = (offsets[c1] + 15) & ~u64(15);
+        j.offs = c.d_offs.as<u32>() + c0; j.n = c1 - c0;
+        j.spans = c.d_spans.as<gm_span>() + c0; j.out = c.d_ids.p; j.cap = cap_ids; j.status = c.d_status.as<int32_t>() + c0;
+        j.trees = trees ? c.d_trees.as<u32>() + c0 : nullptr;
+        j.mode = desc ? MatchJob::DESCRIPTORS : MatchJob::IDS;
+        j.keep_cursor = k != 0;
+        int st = e->enqueue_match(c, j, c.sc);
         if (st != GM_OK) return st;
         CUDA_TRY(cudaMemcpyAsync(&c.h_cur[k], &c.d_ctrl.as<Ctrl>()->cursor, sizeof(u64), cudaMemcpyDeviceToHost, c.sc));
         CUDA_TRY(cudaEventRecord(c.ev_comp[k], c.sc));
@@ -1159,8 +985,10 @@ int32_t gm_retain_match_batch_device(gm_engine* e, const void* d_blob, uint64_t 
     CUDA_TRY(cudaSetDevice(e->device));
     std::lock_guard<std::mutex> gr(e->mu_ret);      // the retained lookup's scratch is engine-wide: one lookup at a time
     { int st = auto_flush(e, true); if (st != GM_OK) return st; }
+    RetainJob j;
+    j.blob = d_blob; j.blob_bytes = blob_bytes; j.offs = d_offs; j.n = n; j.spans = d_spans; j.ids = d_ids; j.cap_ids = std::min<u64>(cap_ids, 0xFFFFFFFFull); j.status = d_status;
     u64 total = 0;
-    int st = e->run_retain(d_blob, blob_bytes, d_offs, n, d_spans, d_ids, std::min<u64>(cap_ids, 0xFFFFFFFFull), d_status, static_cast<cudaStream_t>(stream), &total);
+    int st = e->run_retain(j, static_cast<cudaStream_t>(stream), &total);
     if (st != GM_OK) return st;
     if (needed) *needed = total;
     if (total > 0xFFFFFFFFull) { g_err = "batch produces >= 2^32 ids: split it"; return GM_ERR_TOO_LARGE; }
@@ -1189,9 +1017,11 @@ int32_t gm_retain_match_batch(gm_engine* e, const char* blob, const uint32_t* of
     CUDA_TRY(ri.ensure(std::max<u64>(cap_ids, 1) * sizeof(u32)));
     if (blob_bytes) CUDA_TRY(cudaMemcpyAsync(rb.p, blob, blob_bytes, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(ro.p, offsets, (n + 1) * sizeof(u32), cudaMemcpyHostToDevice, s));
+    RetainJob j;
+    j.blob = rb.p; j.blob_bytes = blob_bytes; j.offs = ro.as<u32>(); j.n = n; j.spans = rs.as<gm_span>(); j.ids = ri.as<u32>();
+    j.cap_ids = std::min<u64>(cap_ids, 0xFFFFFFFFull); j.status = rt.as<int32_t>();
     u64 total = 0;
-    int st = e->run_retain(rb.p, blob_bytes, ro.as<u32>(), n, rs.as<gm_span>(), ri.as<u32>(), std::min<u64>(cap_ids, 0xFFFFFFFFull),
-                           rt.as<int32_t>(), s, &total);
+    int st = e->run_retain(j, s, &total);
     if (st != GM_OK) return st;
     CUDA_TRY(cudaMemcpyAsync(status, rt.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(out_spans, rs.p, n * sizeof(gm_span), cudaMemcpyDeviceToHost, s));
@@ -1450,25 +1280,20 @@ int32_t gm_allgatherv_device(gm_engine* e, const uint32_t* d_index, const gm_spa
 // ---- fused gather over peer memory ------------------------------------------------------------------------------------
 int32_t gm_gather_create(gm_engine* e, uint32_t world, uint32_t rank, uint64_t slab_topics, uint64_t slab_ids, uint8_t* out_handle) {
     if (!e || !out_handle || world == 0 || world > 8 || rank >= world || slab_topics == 0 || slab_ids == 0) return GM_ERR_INVALID_ARG;
-    slab_topics = (slab_topics + 3) & ~uint64_t(3); slab_ids = (slab_ids + 3) & ~uint64_t(3);       // every slab starts on a 16-byte boundary
-    if (slab_ids * world > 0xFFFFFFFFull || slab_topics * world > 0xFFFFFFF0ull) { g_err = "gathered arrays exceed 32-bit offsets"; return GM_ERR_TOO_LARGE; }
+    const GatherLayout layout = gather_layout(world, slab_topics, slab_ids);
+    if (layout.slab_ids * world > 0xFFFFFFFFull || layout.slab_topics * world > 0xFFFFFFF0ull) { g_err = "gathered arrays exceed 32-bit offsets"; return GM_ERR_TOO_LARGE; }
     if (e->flags & GM_FLAG_HOST_ONLY) { g_err = "host-only engine has no device"; return GM_ERR_NO_DEVICE; }
     std::lock_guard<std::mutex> g(e->mu_dev);
     CUDA_TRY(cudaSetDevice(e->device));
     gm_engine::Gather& G = e->gather;
     if (G.block) { g_err = "gm_gather_create: already created (gm_gather_destroy first)"; return GM_ERR_INVALID_ARG; }
-    G.world = world; G.rank = rank; G.slab_topics = slab_topics; G.slab_ids = slab_ids; G.epoch = 0; G.connected = false;
-    const size_t a = 256;
-    G.off_spans = (gm_engine::Gather::off_ids + static_cast<size_t>(world) * slab_ids * 4 + a - 1) / a * a;
-    G.off_index = G.off_spans + static_cast<size_t>(world) * slab_topics * 8;
-    G.off_counts = (G.off_index + static_cast<size_t>(world) * slab_topics * 4 + a - 1) / a * a;
-    G.off_flags = G.off_counts + static_cast<size_t>(world) * 16;
-    G.bytes = G.off_flags + 256;
+    static_cast<GatherLayout&>(G) = layout;
+    G.rank = rank; G.epoch = 0; G.connected = false;
     void* p = nullptr;
     CUDA_TRY(cudaMalloc(&p, G.bytes));
     G.block = static_cast<char*>(p);
     CUDA_TRY(cudaMemset(G.block + G.off_counts, 0, G.bytes - G.off_counts));
-    const unsigned long long geo[3] = {world, slab_topics, slab_ids};       // the layout must be the same on every rank: checked at connect
+    const unsigned long long geo[3] = {world, G.slab_topics, G.slab_ids};       // the layout must be the same on every rank: checked at connect
     CUDA_TRY(cudaMemcpy(G.block, geo, sizeof(geo), cudaMemcpyHostToDevice));
     CUDA_TRY(cudaDeviceSynchronize());
     cudaIpcMemHandle_t h;
@@ -1519,26 +1344,19 @@ int32_t gm_match_gather_device(gm_engine* e, const void* d_blob, uint64_t blob_b
     { int st = auto_flush(e); if (st != GM_OK) return st; }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     std::lock_guard<std::mutex> gd(e->mu_dev);
-    int st = e->enqueue_match(e->devctx, d_blob, blob_bytes, d_offsets, n, nullptr, nullptr, G.slab_ids, nullptr, d_status, s, false, false, false, d_sel, 0, nullptr, true, 0,
-                              nullptr, true);
+    MatchJob j;
+    j.blob = d_blob; j.blob_bytes = blob_bytes; j.offs = d_offsets; j.sel = d_sel; j.n = n; j.cap = G.slab_ids; j.status = d_status;
+    j.mode = MatchJob::GATHER; j.gather = &G; j.blocks = G.peer; j.rank = G.rank;
+    int st = e->enqueue_match(e->devctx, j, s);
     if (st != GM_OK) return st;
     // contribution (rows, ids) into every rank's counts + the epoch barrier: when it has passed on a rank, all ranks' data is there
     G.epoch++;
     const unsigned long long* d_m = n ? &e->devctx.d_ctrl.as<Ctrl>()->cursor : nullptr;
     if (!d_m) { CUDA_TRY(e->devctx.d_ctrl.ensure(sizeof(Ctrl))); CUDA_TRY(cudaMemsetAsync(e->devctx.d_ctrl.p, 0, sizeof(Ctrl), s)); d_m = &e->devctx.d_ctrl.as<Ctrl>()->cursor; }
     void** dp = G.d_ptrs.as<void*>();
-    if (!e->knobs.gather_direct && G.world > 1) {
-        k_gather_push<<<e->num_sms * 4, 256, 0, s>>>(reinterpret_cast<char* const*>(dp + 16), G.rank, G.world, gm_engine::Gather::off_ids, G.off_spans, G.off_index,
-                                                     G.rank * G.slab_topics, G.rank * G.slab_ids, n, d_m);
-        e->launches++;
-    }
-    // the error word reports on THIS step only: a straggler of an earlier step (a rank that arrived after the bounded wait) must not
-    // make every later gm_gather_get fail (only this rank's own k_gather_finish ever writes the word)
-    CUDA_TRY(cudaMemsetAsync(reinterpret_cast<u32*>(G.block + G.off_flags) + 32, 0, sizeof(u32), s));
-    k_gather_finish<<<1, 32, 0, s>>>(reinterpret_cast<unsigned long long* const*>(dp), reinterpret_cast<u32* const*>(dp + 8), reinterpret_cast<u32*>(G.block + G.off_flags),
-                                     G.rank, G.world, n, d_m, G.epoch, reinterpret_cast<u32*>(G.block + G.off_flags) + 32);
-    e->launches++;
-    CUDA_TRY(cudaGetLastError());
+    CudaLauncher l{s, nullptr, &e->ring_n, &e->launches};
+    if ((st = gather_push(l, G, e->knobs.gather_direct, static_cast<u32>(e->num_sms), reinterpret_cast<char* const*>(dp + 16), G.rank, n, d_m)) != GM_OK) return st;
+    if ((st = gather_finish(l, G, G.block, reinterpret_cast<unsigned long long* const*>(dp), reinterpret_cast<u32* const*>(dp + 8), G.rank, n, d_m, G.epoch)) != GM_OK) return st;
     CUDA_TRY(cudaEventRecord(e->devctx.ev_done, s));
     e->devctx.recorded = true;
     return GM_OK;
@@ -1552,7 +1370,7 @@ int32_t gm_gather_get(gm_engine* e, gm_gather_view* out, void* stream) {
     CUDA_TRY(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
     u32 err = 0;
     CUDA_TRY(cudaMemcpy(&err, G.block + G.off_flags + 32 * 4, 4, cudaMemcpyDeviceToHost));
-    out->d_ids = reinterpret_cast<const uint32_t*>(G.block + gm_engine::Gather::off_ids); out->d_spans = reinterpret_cast<const gm_span*>(G.block + G.off_spans);
+    out->d_ids = reinterpret_cast<const uint32_t*>(G.block + GatherLayout::off_ids); out->d_spans = reinterpret_cast<const gm_span*>(G.block + G.off_spans);
     out->d_index = reinterpret_cast<const uint32_t*>(G.block + G.off_index); out->d_counts = reinterpret_cast<const uint64_t*>(G.block + G.off_counts);
     out->slab_topics = G.slab_topics; out->slab_ids = G.slab_ids; out->world = G.world; out->rank = G.rank;
     if (err) { g_err = "fused gather: a rank did not reach the end-of-step barrier"; return GM_ERR_COMM; }

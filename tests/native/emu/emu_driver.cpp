@@ -1,7 +1,9 @@
-// TEST INFRASTRUCTURE: the match and retained-lookup pipelines of engine.cu (enqueue_match / enqueue_retain) over HOST
-// memory, with the REAL kernel sources (kernels.cuh, retain_kernels.cuh, relations.cuh compiled with -DGM_CPU_EMU) run
-// by the CPU emulation in cuda_runtime.h.  Exposed as a small C interface for tests/test_emu_kernels.py, which compares
-// the results with the oracle.  Build (tests/test_emu_kernels.py does it):
+// TEST INFRASTRUCTURE: the engine's own match, fused-gather and retained-lookup pipelines and its flush shipping policy
+// (rmqtt_b200/csrc/pipeline.h, which engine.cu runs on the device) over HOST memory, with the REAL kernel sources
+// (kernels.cuh, retain_kernels.cuh, comm.cuh, relations.cuh compiled with -DGM_CPU_EMU) run by the CPU emulation in
+// cuda_runtime.h.  This file supplies only how an operation is carried out there: a launcher (emu::launch, std::memset),
+// a shipper into a byte image of every table, and host buffers for the scratch the pipelines size.  Exposed as a small C
+// interface for tests/test_emu_kernels.py, which compares the results with the oracle.  Build (tests/test_emu_kernels.py does it):
 //   g++ -O1 -g -std=c++17 -DGM_CPU_EMU -Itests/native/emu -Irmqtt_b200/csrc -shared -fPIC tests/native/emu/emu_driver.cpp \
 //       rmqtt_b200/csrc/host_trie.cpp rmqtt_b200/csrc/retain_tree.cpp -o <out>.so     (+ -fsanitize=address,undefined for the ASan run)
 #include <cuda_runtime.h>      // the emulation (this directory is first on the include path)
@@ -10,129 +12,108 @@
 #include <vector>
 
 #include "../../../include/gpumqtt.h"
-#include "comm.cuh"
-#include "host_trie.h"
-#include "kernels.cuh"
+#include "pipeline.h"
 #include "relations.cuh"
-#include "retain_kernels.cuh"
-#include "retain_tree.h"
 
 using namespace gm;
 
 namespace {
 
-struct Ctrl { unsigned long long cursor; unsigned long long stats[24]; u32 slow_count; u32 tile_counter; };   // engine.cu's control block
-
-constexpr int K2_FAST_L = 8, K2_THREADS = 512, K2_CTAS_PER_SM = 3;
 constexpr u32 EMU_SMS = 2;               // the emulated part has two SMs: several CTAs per kernel, dynamic tile hand-out exercised
 
-// A "device copy" of one table, maintained ONLY by what gm_engine::flush_impl would ship (engine.cu upload_table /
-// upload_appendable / stage_patches): whole arrays after a re-hash or for the first shipment, appended tails, and the slots the
-// host mirror listed as dirty.  A slot the mirror changed without listing it stays stale here — and shows up as a wrong match.
-template <class T> struct ImgBuf {
-    std::vector<T> v;                    // v.size() plays the role of DevBuf::cap (elements)
-    size_t up = 0;                       // shipped up to here (appendable arrays) / shipped size (tables)
-    bool have = false;
-    template <class H> void fresh(const H& host, size_t min_elems) {
-        v.assign(std::max(std::max(host.size(), min_elems), size_t(8)), T{});
-        std::memset(static_cast<void*>(v.data()), 0xCD, v.size() * sizeof(T));          // never-shipped bytes are garbage on a device
-        if (host.size()) std::memcpy(static_cast<void*>(v.data()), host.data(), host.size() * sizeof(T));
-        up = host.size(); have = true;
+// host stand-in for a cudaMalloc'd buffer: 256-byte aligned, whole 256-byte units
+struct Bytes {
+    struct alignas(256) Unit { unsigned char b[256]; };
+    std::vector<Unit> v;
+    Bytes() = default;
+    Bytes(size_t bytes, int fill) { alloc(bytes, fill); }
+    void alloc(size_t bytes, int fill) {
+        v.assign((bytes + 255) / 256, Unit{});
+        if (!v.empty()) std::memset(static_cast<void*>(v.data()), fill, v.size() * sizeof(Unit));
     }
-    template <class H> void patch(const H& host, std::vector<u32>& dirty) {
-        for (u32 i : dirty) v[i] = host[i];
+    template <class T> T* as() { return v.empty() ? nullptr : reinterpret_cast<T*>(v.data()); }
+    size_t cap() const { return v.size() * sizeof(Unit); }
+};
+
+// pipeline.h's launcher: kernels run to completion one after the other, on the calling thread
+struct EmuLauncher {
+    template <class... P, class... A>
+    int launch(void (*k)(P...), u32 grid, u32 block, size_t, A... a) {
+        emu::launch(dim3(grid), dim3(block), [&] { k(a...); });
+        return GM_OK;
+    }
+    int memset(void* p, int v, size_t bytes) { std::memset(p, v, bytes); return GM_OK; }
+    int copy(void* dst, const void* src, size_t bytes) { std::memcpy(dst, src, bytes); return GM_OK; }
+    int mark(int) { return GM_OK; }
+};
+
+// pipeline.h's shipper into a byte image per table: a slot the host mirror changed without listing it as dirty stays
+// stale there — and shows up as a wrong match.  Bytes never shipped read 0xCD (garbage, as on a device).
+struct ImageShipper {
+    int fresh(Bytes& b, const void* src, size_t bytes, size_t cap_bytes) {
+        b.alloc(cap_bytes, 0xCD);
+        if (bytes) std::memcpy(b.as<char>(), src, bytes);
+        return GM_OK;
+    }
+    int append(Bytes& b, size_t off, const void* src, size_t bytes) { std::memcpy(b.as<char>() + off, src, bytes); return GM_OK; }
+    template <class V>
+    int patch(Bytes& b, const V& host, std::vector<u32>& dirty) {
+        using T = elem_t<V>;
+        for (u32 i : dirty) std::memcpy(b.as<char>() + static_cast<size_t>(i) * sizeof(T), &host[i], sizeof(T));
         dirty.clear();
+        return GM_OK;
     }
-    template <class H> void table(const H& host, bool& full, std::vector<u32>& dirty) {       // engine.cu upload_table
-        if (full || !have || up != host.size() || dirty.size() * 8 > host.size()) { fresh(host, 0); dirty.clear(); }
-        else patch(host, dirty);
-        full = false;
-    }
-    template <class H> void appendable(const H& host, std::vector<u32>* dirty) {              // engine.cu upload_appendable
-        if ((up == 0 && (host.size() > 0 || !have)) || host.size() > v.size()) { fresh(host, std::max(host.size() * 2, size_t(1024))); if (dirty) dirty->clear(); return; }
-        const size_t before = up;
-        if (host.size() > up) { std::memcpy(static_cast<void*>(v.data() + up), host.data() + up, (host.size() - up) * sizeof(T)); up = host.size(); }
-        if (dirty) {
-            dirty->erase(std::remove_if(dirty->begin(), dirty->end(), [&](u32 i) { return i >= before; }), dirty->end());
-            patch(host, *dirty);
-        }
+    size_t capacity(const Bytes& b) const { return b.cap(); }
+};
+
+struct MatchBufs {                       // the scratch of one match, as plan_match sized it
+    Bytes tok, tok8, meta, slow, ctrl, sort, hist, gstack, gpool;
+    explicit MatchBufs(const MatchPlan& p)
+        : tok(p.tok, 0), tok8(p.tok8, 0), meta(p.meta, 0), slow(p.slow, 0), ctrl(p.ctrl, 0), sort(p.sort, 0), hist(p.hist, 0), gstack(p.gstack, 0), gpool(p.gpool, 0) {}
+    MatchScratch scratch() {
+        return {tok.as<u32>(), tok8.as<u32>(), meta.as<u32>(), slow.as<u32>(), ctrl.as<Ctrl>(), sort.as<u32>(), hist.as<u32>(), gstack.as<u64>(), gpool.as<Desc>()};
     }
 };
 
 struct EmuEngine {
     HostTrie trie{128};
     RetainTreeHost rtree{&trie};
-    u32 pool_rows = 24;                  // engine.cu K2_POOL_ROWS (tests lower it to push topics onto the deferred kernel)
-    u32 site_bits = 10;
+    u32 pool_rows = K2_POOL_ROWS;        // (tests lower it to push topics onto the deferred kernel)
     // optional device image (emu_use_image): the kernels then read copies that only flush() updates
     bool image = false, manual_flush = false;
-    ImgBuf<EdgeSlot> i_edges; ImgBuf<DictSlot> i_dict; ImgBuf<Range> i_ranges; ImgBuf<u32> i_values, i_cfilter, i_tree_slots, i_rvals; ImgBuf<u8> i_pool;
-    ImgBuf<RKid> i_rkids; ImgBuf<REdge> i_redges;
-    u64 up_values_epoch = 0;
+    Bytes d_edges, d_dict, d_ranges, d_values, d_pool, d_cfilter, d_tree_slots, d_rnodes, d_rkids, d_redges, d_rvals;
+    ShipMarks up;
     TrieView dev_view{}; RetainView dev_rview{};
-    u64 flushes = 0;
 
-    bool flush() {                       // engine.cu gm_engine::flush_impl, shipping policy only
-        if (!trie.any_dirty() && !rtree.dirty && flushes) return true;
+    bool flush() {                       // gm_engine::flush_impl, into the image
+        if (!trie.any_dirty() && !rtree.dirty) return true;
         if (!trie.sync()) return false;
-        if (trie.values_epoch != up_values_epoch) { i_values.up = i_ranges.up = 0; up_values_epoch = trie.values_epoch; }
-        if (rtree.dirty || !flushes) {
-            rtree.prepare_flush();
-            if (rtree.full || !i_rkids.have) { i_rkids.fresh(rtree.rkids, rtree.rkids.size() + rtree.rkids.size() / 4 + 1024); i_redges.fresh(rtree.redges, 0); i_rvals.fresh(rtree.rvals, rtree.rvals.size() + 1024); }
-            else {
-                bool full_edges = false;
-                i_rkids.appendable(rtree.rkids, &rtree.dirty_kids);
-                i_redges.table(rtree.redges, full_edges, rtree.dirty_edges);
-                i_rvals.appendable(rtree.rvals, &rtree.dirty_vals);
-            }
-            rtree.shipped();
-        }
-        i_edges.table(trie.edges, trie.full_edges, trie.dirty_edges);
-        i_dict.table(trie.dict, trie.full_dict, trie.dirty_dict);
-        i_ranges.appendable(trie.ranges, nullptr);
-        i_values.appendable(trie.values, nullptr);
-        i_pool.appendable(trie.pool, nullptr);
-        if (trie.cfilter_dirty || !i_cfilter.have) { i_cfilter.fresh(trie.cfilter, 0); trie.cfilter_dirty = false; }
-        if (trie.trees_dirty || !i_tree_slots.have) { i_tree_slots.fresh(trie.tree_slots, 0); trie.trees_dirty = false; }
-        trie.root_dirty = false;
-        dev_view = host_view();
-        dev_view.edges = i_edges.v.data(); dev_view.ranges = i_ranges.v.data(); dev_view.values = i_values.v.data(); dev_view.dict = i_dict.v.data();
-        dev_view.pool = i_pool.v.data(); dev_view.cfilter = i_cfilter.v.data(); dev_view.tree_slots = i_tree_slots.v.data();
-        dev_rview = host_rview();
-        dev_rview.kids = i_rkids.v.data(); dev_rview.edges = i_redges.v.data(); dev_rview.vals = i_rvals.v.data();
-        flushes++;
+        ImageShipper sh;
+        bool r_shipped = false;
+        ship(sh, TableBufs<Bytes>{&d_edges, &d_dict, &d_ranges, &d_values, &d_pool, &d_cfilter, &d_tree_slots, &d_rnodes, &d_rkids, &d_redges, &d_rvals},
+             trie, rtree, up, &r_shipped);
+        dev_view = make_trie_view(trie, {d_edges.as<EdgeSlot>(), d_ranges.as<Range>(), d_values.as<u32>(), d_dict.as<DictSlot>(), d_pool.as<u8>(),
+                                         d_cfilter.as<u32>(), d_tree_slots.as<u32>()});
+        dev_rview = make_retain_view(rtree, {d_rkids.as<RKid>(), d_redges.as<REdge>(), d_rvals.as<u32>()});
+        if (r_shipped) rtree.shipped();
         return true;
     }
-    // what a match sees: the live host arrays, or — with the device image — the copies as of the last flush (auto-flush engines
-    // flush before every match, GM_FLAG_MANUAL_FLUSH ones only when told to)
+    // what a match sees: the live host arrays, or — with the device image — the copies as of the last flush (engine.cu
+    // auto_flush: GM_FLAG_MANUAL_FLUSH engines flush only when told to, once the tables they need were shipped)
     bool prepare(bool retained) {
         if (!image) { if (!trie.sync()) return false; if (retained) { rtree.prepare_flush(); rtree.shipped(); } return true; }
-        if (!manual_flush || !flushes) return flush();
-        return true;
+        if (manual_flush && d_edges.cap() && (!retained || d_rnodes.cap())) return true;
+        return flush();
     }
-    TrieView view() { return image ? dev_view : host_view(); }
-    RetainView rview() { return image ? dev_rview : host_rview(); }
-
-    TrieView host_view() {               // engine.cu gm_engine::view(), host pointers instead of device pointers
-        TrieView v{};
-        v.edges = trie.edges.data(); v.ranges = trie.ranges.data(); v.values = trie.values.data(); v.dict = trie.dict.data(); v.pool = trie.pool.data();
-        v.cfilter = trie.cfilter.data(); v.cfilter_mask = static_cast<u32>(trie.cfilter.size() - 1);
-        v.edge_mask = static_cast<u32>(trie.edges.size() - 1);
-        v.win_mask = trie.win_mask(); v.win_shift = trie.win_shift(); v.nwin_mask = trie.nwin_mask();
-        v.dict_mask = static_cast<u32>(trie.dict.size() - 1);
-        v.root_plus = trie.root_plus; v.root_hash_ref = trie.root_hash_ref; v.root_hash_cnt = trie.root_hash_cnt; v.root_mask = trie.root_mask;
-        v.max_depth = trie.max_depth;
-        v.tree_slots = trie.tree_slots.data(); v.n_trees = static_cast<u32>(trie.tree_slots.size());
-        return v;
+    TrieView view() {
+        if (image) return dev_view;
+        return make_trie_view(trie, {trie.edges.data(), trie.ranges.data(), trie.values.data(), trie.dict.data(), trie.pool.data(), trie.cfilter.data(), trie.tree_slots.data()});
     }
-    RetainView host_rview() {            // engine.cu gm_engine::rview()
-        RetainView v{};
-        v.kids = rtree.rkids.data(); v.edges = rtree.redges.data(); v.vals = rtree.rvals.data();
-        v.edge_mask = static_cast<u32>(rtree.redges.size() - 1);
-        if (!rtree.rnodes.empty()) { v.root_first_kid = rtree.rnodes[0].first_kid; v.root_nk_flags = rtree.rnodes[0].nkids | (rtree.rnodes[0].flags << 28); }
-        v.root_plain_kids = rtree.root_plain_kids; v.root_plain_val_hi = rtree.root_plain_val_hi; v.max_depth = rtree.max_depth;
-        v.n_kids = static_cast<u32>(rtree.rkids.size());
-        return v;
+    RetainView rview() { return image ? dev_rview : make_retain_view(rtree, {rtree.rkids.data(), rtree.redges.data(), rtree.rvals.data()}); }
+    MatchGeometry geometry(bool tok_bulk) const {
+        MatchGeometry g;
+        g.num_sms = EMU_SMS; g.pool_rows = pool_rows; g.site_bits = 10; g.tok_bulk = tok_bulk;
+        return g;
     }
 };
 
@@ -153,8 +134,7 @@ int32_t emu_compact(void* h) {           // gm_compact: dictionary + value compa
     std::vector<u32> remap;
     e->trie.compact(&keep, &remap);
     e->rtree.remap_tokens(remap);
-    e->i_ranges.up = e->i_values.up = e->i_pool.up = 0; e->up_values_epoch = e->trie.values_epoch;
-    e->i_edges.have = e->i_dict.have = false;
+    e->up.forget_trie(e->trie.values_epoch);
     return 0;
 }
 
@@ -185,7 +165,7 @@ uint64_t emu_retain_bulk_load(void* h, const char* blob, const uint32_t* offs, c
     return static_cast<EmuEngine*>(h)->rtree.set_batch(blob, offs, vals, n);
 }
 
-// Router::matches for a batch through k_tokenize -> k_bucket_scan -> k_bucket_scatter -> k_match_fast -> k_match_slow.
+// Router::matches for a batch through the match pipeline.
 // flags: bit 0 descriptor mode (the descriptors are expanded here from the host mirror, so `out_ids` holds ids either way),
 //        bit 1 the bulk-staged tokeniser, bit 2 the instrumented (STATS) instantiations; work[4] = V, E, F, M then.
 // Returns 0, or -3 with *needed when cap_ids is too small (the engine's capacity protocol).
@@ -205,7 +185,6 @@ int32_t emu_match_ex(void* h, const char* blob_in, const uint32_t* offs, uint64_
     const u32 blob_bytes = offs[n_entries];
     const u32 n = graph_form ? n_real + 37u : n_real;            // launch size (rows beyond the real batch must stay untouched)
     u32 hdr_store[4] = {n_real, blob_bytes, 0u, 0u};
-    const u32* hdr = graph_form ? hdr_store : nullptr;
     std::vector<u32> offs_cap;
     if (graph_form) {                                             // the in-block holds capacity + 1 offsets; the tail is never read
         offs_cap.assign(offs, offs + n_entries + 1);
@@ -214,66 +193,34 @@ int32_t emu_match_ex(void* h, const char* blob_in, const uint32_t* offs, uint64_
     }
     // the bulk stage wants a 16-byte aligned blob that may be read up to a 16-byte boundary
     const size_t readable = (static_cast<size_t>(blob_bytes) + 15) & ~size_t(15);
-    std::vector<u8> blob_store(readable + 64, 0);
-    u8* blob = blob_store.data() + ((16 - (reinterpret_cast<uintptr_t>(blob_store.data()) & 15)) & 15);
-    std::memcpy(blob, blob_in, blob_bytes);
-    const u32 S = std::max<u32>(1u, tv.max_depth);
-    std::vector<u32> tok(S > TOK8 ? static_cast<size_t>(S) * n : 64), meta(n), slow(n);
-    std::vector<u32> tok8_store(static_cast<size_t>(n) * TOK8 + 16), sort_store(static_cast<size_t>(n) * 11 + 64);
-    u32* tok8 = tok8_store.data() + ((32 - (reinterpret_cast<uintptr_t>(tok8_store.data()) & 31)) & 31) / 4;
-    u32* sortb = sort_store.data() + ((32 - (reinterpret_cast<uintptr_t>(sort_store.data()) & 31)) & 31) / 4;
-    Ctrl ctrl{};
-    const u32 NB = 1u << e.site_bits;
-    std::vector<u32> hist_store(2 * static_cast<size_t>(NB) + 16, 0);
-    u32* hist = hist_store.data() + ((16 - (reinterpret_cast<uintptr_t>(hist_store.data()) & 15)) & 15) / 4;
-    u32* bcursor = hist + NB;
-    u32* bkey = sortb; u32* perm = bkey + n; u32* meta_sorted = perm + n;
-    u32* tok8_sorted = meta_sorted + n + ((8 - (3 * static_cast<size_t>(n)) % 8) % 8);
-    const u32 stack_cap = 32u * (tv.max_depth + 2u) + 64u;
-    const int k3_blocks = EMU_SMS * 4;
-    std::vector<u64> gstack(static_cast<size_t>(k3_blocks) * 8 * stack_cap);
-    const int k2_grid = EMU_SMS * K2_CTAS_PER_SM;
-    std::vector<Desc> gpool(static_cast<size_t>(k2_grid) * K2_THREADS * std::max<u32>(e.pool_rows, 1u));
+    Bytes blob(readable + 64, 0);
+    std::memcpy(blob.as<char>(), blob_in, blob_bytes);
     std::vector<uint2> descs;
     std::vector<u32> ids_tmp;
     void* d_out = out_ids;
-    u64 cap = cap_ids;
     if (desc) { descs.resize(cap_ids + 1); d_out = descs.data(); }
-
     std::vector<int32_t> status_cap;
     int32_t* status_k = status;
     if (graph_form) { status_cap.assign(n, 0x7F7F7F7F); status_k = status_cap.data(); }
     for (u32 i = 0; i < n_real; ++i) status[i] = 0x7F7F7F7F;   // every row must be written by the tokeniser
-    emu::launch(dim3((n + TOK_THREADS - 1) / TOK_THREADS), dim3(TOK_THREADS), [&] {
-        if (bulk) k_tokenize<true>(blob, blob_bytes, static_cast<u32>(readable), offs, sel, n, hdr, tv, S, tok8, tok.data(), meta.data(), status_k, bkey, hist, e.site_bits, 0u);
-        else k_tokenize<false>(blob, blob_bytes, static_cast<u32>(readable), offs, sel, n, hdr, tv, S, tok8, tok.data(), meta.data(), status_k, bkey, hist, e.site_bits, 0u);
-    });
-    emu::launch(dim3(1), dim3(1024), [&] { k_bucket_scan(hist, bcursor, NB); });
-    emu::launch(dim3((n + 255) / 256), dim3(256), [&] { k_bucket_scatter(bkey, bcursor, n, hdr, perm, tok8, meta.data(), tok8_sorted, meta_sorted); });
-    if (graph_form) {
-        for (u32 i = n_real; i < n; ++i) if (status_cap[i] != 0x7F7F7F7F) return -50;      // a row beyond the real batch was touched
-        std::memcpy(status, status_cap.data(), n_real * sizeof(int32_t));
-    }
     std::vector<gm_span> spans_cap;
     gm_span* spans_k = out_spans;
     if (graph_form) { spans_cap.assign(n, gm_span{0xABABABABu, 0xABABABABu}); spans_k = spans_cap.data(); }
 
-    MatchParams mp{};
-    mp.tv = tv; mp.tok8 = tok8; mp.tok = tok.data(); mp.meta = meta.data(); mp.n = n; mp.n_ptr = hdr; mp.tok_levels = S;
-    mp.spans = reinterpret_cast<uint2*>(spans_k); mp.out_ids = static_cast<u32*>(d_out); mp.out_desc = static_cast<uint2*>(d_out); mp.cap_ids = cap;
-    mp.status = status_k; mp.trees = trees;
-    mp.cursor = &ctrl.cursor; mp.slow_list = slow.data(); mp.slow_count = &ctrl.slow_count; mp.tile_counter = &ctrl.tile_counter; mp.stats = ctrl.stats;
-    mp.perm = perm; mp.tok8_sorted = tok8_sorted; mp.meta_sorted = meta_sorted;
-    mp.flags = MP_SORTED_ROWS; mp.tile_chunk = 1;
-    emu::launch(dim3(k2_grid), dim3(K2_THREADS), [&] {
-        if (stats) { if (desc) k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, true, true>(mp, gpool.data(), e.pool_rows); else k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, true, false>(mp, gpool.data(), e.pool_rows); }
-        else { if (desc) k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, true>(mp, gpool.data(), e.pool_rows); else k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, false>(mp, gpool.data(), e.pool_rows); }
-    });
-    emu::launch(dim3(k3_blocks), dim3(256), [&] {
-        if (stats) { if (desc) k_match_slow<true, true>(mp, gstack.data(), stack_cap); else k_match_slow<true, false>(mp, gstack.data(), stack_cap); }
-        else { if (desc) k_match_slow<false, true>(mp, gstack.data(), stack_cap); else k_match_slow<false, false>(mp, gstack.data(), stack_cap); }
-    });
+    MatchJob j;
+    j.blob = blob.as<u8>(); j.blob_bytes = blob_bytes; j.readable_bytes = readable; j.offs = offs; j.sel = sel; j.n = n; j.hdr = graph_form ? hdr_store : nullptr;
+    j.spans = spans_k; j.out = d_out; j.cap = cap_ids; j.status = status_k; j.trees = trees;
+    j.mode = desc ? MatchJob::DESCRIPTORS : MatchJob::IDS;
+    j.stats = stats;
+    const MatchGeometry g = e.geometry(bulk);
+    const MatchPlan p = plan_match(g, j, tv.max_depth);
+    MatchBufs m(p);
+    EmuLauncher l;
+    match_pipeline(l, g, j, p, tv, m.scratch());
+    const Ctrl& ctrl = *m.ctrl.as<Ctrl>();
     if (graph_form) {
+        for (u32 i = n_real; i < n; ++i) if (status_cap[i] != 0x7F7F7F7F) return -50;      // a row beyond the real batch was touched
+        std::memcpy(status, status_cap.data(), n_real * sizeof(int32_t));
         for (u32 i = n_real; i < n; ++i) if (spans_cap[i].off != 0xABABABABu) return -51;
         std::memcpy(out_spans, spans_cap.data(), n_real * sizeof(gm_span));
     }
@@ -293,7 +240,7 @@ int32_t emu_match_ex(void* h, const char* blob_in, const uint32_t* offs, uint64_
             else {
                 u64 o = d.x, c = d.y;
                 if (d.y == CNT_BIG) { o = e.trie.ranges[d.x].off; c = e.trie.ranges[d.x].cnt; }
-                for (u64 j = 0; j < c; ++j) ids_tmp.push_back(e.trie.values[o + j]);
+                for (u64 q = 0; q < c; ++q) ids_tmp.push_back(e.trie.values[o + q]);
             }
         }
         w = ids_tmp.size();
@@ -322,29 +269,19 @@ int32_t emu_partition(const char* blob, const uint32_t* offs, uint64_t n, uint32
 }
 
 // ---- the fused gather over "peer memory": every rank's block lives in host memory of this one process ---------------------------
-struct GatherWorld {
-    u32 world = 0; u64 slab_topics = 0, slab_ids = 0;
-    static constexpr size_t off_ids = 256;
-    size_t off_spans = 0, off_index = 0, off_counts = 0, off_flags = 0, bytes = 0;
-    std::vector<std::vector<char>> store;
+struct GatherWorld : GatherLayout {
+    std::vector<Bytes> store;
     std::vector<char*> block;
     std::vector<u32> epoch;
     std::vector<unsigned long long> cursor;      // the match cursor of every rank's last step (k_gather_push / k_gather_finish read it)
 };
-void* emu_gather_new(uint32_t world, uint64_t slab_topics, uint64_t slab_ids) {       // engine.cu gm_gather_create's layout
+void* emu_gather_new(uint32_t world, uint64_t slab_topics, uint64_t slab_ids) {       // gm_gather_create
     GatherWorld* g = new GatherWorld();
-    slab_topics = (slab_topics + 3) & ~uint64_t(3); slab_ids = (slab_ids + 3) & ~uint64_t(3);
-    g->world = world; g->slab_topics = slab_topics; g->slab_ids = slab_ids;
-    const size_t a = 256;
-    g->off_spans = (GatherWorld::off_ids + static_cast<size_t>(world) * slab_ids * 4 + a - 1) / a * a;
-    g->off_index = g->off_spans + static_cast<size_t>(world) * slab_topics * 8;
-    g->off_counts = (g->off_index + static_cast<size_t>(world) * slab_topics * 4 + a - 1) / a * a;
-    g->off_flags = g->off_counts + static_cast<size_t>(world) * 16;
-    g->bytes = g->off_flags + 256;
+    static_cast<GatherLayout&>(*g) = gather_layout(world, slab_topics, slab_ids);
     g->store.resize(world); g->block.resize(world); g->epoch.assign(world, 0); g->cursor.assign(world, 0);
     for (u32 w = 0; w < world; ++w) {
-        g->store[w].assign(g->bytes + 256, static_cast<char>(0xEE));        // (stale bytes must never be read as results)
-        g->block[w] = g->store[w].data() + ((256 - (reinterpret_cast<uintptr_t>(g->store[w].data()) & 255)) & 255);
+        g->store[w].alloc(g->bytes, 0xEE);                                  // (stale bytes must never be read as results)
+        g->block[w] = g->store[w].as<char>();
         std::memset(g->block[w] + g->off_counts, 0, g->bytes - g->off_counts);
     }
     return g;
@@ -367,57 +304,22 @@ int32_t emu_match_gather(void* gw, uint32_t rank, void* h, const char* blob_in, 
         const TrieView tv = e.view();
         const u32 blob_bytes = offs[n_entries];
         const size_t readable = (static_cast<size_t>(blob_bytes) + 15) & ~size_t(15);
-        std::vector<u8> blob_store(readable + 64, 0);
-        u8* blob = blob_store.data() + ((16 - (reinterpret_cast<uintptr_t>(blob_store.data()) & 15)) & 15);
-        std::memcpy(blob, blob_in, blob_bytes);
-        const u32 S = std::max<u32>(1u, tv.max_depth);
-        std::vector<u32> tok(S > TOK8 ? static_cast<size_t>(S) * n : 64), meta(n), slow(n);
-        std::vector<u32> tok8_store(static_cast<size_t>(n) * TOK8 + 16), sort_store(static_cast<size_t>(n) * 11 + 64);
-        u32* tok8 = tok8_store.data() + ((32 - (reinterpret_cast<uintptr_t>(tok8_store.data()) & 31)) & 31) / 4;
-        u32* sortb = sort_store.data() + ((32 - (reinterpret_cast<uintptr_t>(sort_store.data()) & 31)) & 31) / 4;
-        Ctrl ctrl{};
-        const u32 NB = 1u << e.site_bits;
-        std::vector<u32> hist_store(2 * static_cast<size_t>(NB) + 16, 0);
-        u32* hist = hist_store.data() + ((16 - (reinterpret_cast<uintptr_t>(hist_store.data()) & 15)) & 15) / 4;
-        u32* bcursor = hist + NB;
-        u32* bkey = sortb; u32* perm = bkey + n; u32* meta_sorted = perm + n;
-        u32* tok8_sorted = meta_sorted + n + ((8 - (3 * static_cast<size_t>(n)) % 8) % 8);
-        const u32 stack_cap = 32u * (tv.max_depth + 2u) + 64u;
-        const int k3_blocks = EMU_SMS * 4, k2_grid = EMU_SMS * K2_CTAS_PER_SM;
-        std::vector<u64> gstack(static_cast<size_t>(k3_blocks) * 8 * stack_cap);
-        std::vector<Desc> gpool(static_cast<size_t>(k2_grid) * K2_THREADS * std::max<u32>(e.pool_rows, 1u));
-        emu::launch(dim3((n + TOK_THREADS - 1) / TOK_THREADS), dim3(TOK_THREADS), [&] {
-            k_tokenize<false>(blob, blob_bytes, static_cast<u32>(readable), offs, sel, n, nullptr, tv, S, tok8, tok.data(), meta.data(), status, bkey, hist, e.site_bits, 0u);
-        });
-        emu::launch(dim3(1), dim3(1024), [&] { k_bucket_scan(hist, bcursor, NB); });
-        emu::launch(dim3((n + 255) / 256), dim3(256), [&] { k_bucket_scatter(bkey, bcursor, n, nullptr, perm, tok8, meta.data(), tok8_sorted, meta_sorted); });
-        MatchParams mp{};
-        mp.tv = tv; mp.tok8 = tok8; mp.tok = tok.data(); mp.meta = meta.data(); mp.n = n; mp.tok_levels = S;
-        mp.cap_ids = G.slab_ids; mp.status = status;
-        mp.cursor = &ctrl.cursor; mp.slow_list = slow.data(); mp.slow_count = &ctrl.slow_count; mp.tile_counter = &ctrl.tile_counter; mp.stats = ctrl.stats;
-        mp.perm = perm; mp.tok8_sorted = tok8_sorted; mp.meta_sorted = meta_sorted;
-        mp.flags = MP_SORTED_ROWS; mp.tile_chunk = 1;
-        mp.g_base_topics = static_cast<u32>(rank * G.slab_topics); mp.g_base_ids = rank * G.slab_ids; mp.g_sel = sel;     // engine.cu enqueue_match, gather_mode
-        if (direct) {
-            mp.g_world = G.world;
-            for (u32 w = 0; w < G.world; ++w) {
-                mp.g_ids[w] = reinterpret_cast<u32*>(G.block[w] + GatherWorld::off_ids); mp.g_spans[w] = reinterpret_cast<uint2*>(G.block[w] + G.off_spans);
-                mp.g_index[w] = reinterpret_cast<u32*>(G.block[w] + G.off_index);
-            }
-        } else {
-            mp.g_world = 1;
-            mp.g_ids[0] = reinterpret_cast<u32*>(G.block[rank] + GatherWorld::off_ids); mp.g_spans[0] = reinterpret_cast<uint2*>(G.block[rank] + G.off_spans);
-            mp.g_index[0] = reinterpret_cast<u32*>(G.block[rank] + G.off_index);
-        }
-        emu::launch(dim3(k2_grid), dim3(K2_THREADS), [&] { k_match_fast<K2_FAST_L, K2_THREADS, K2_CTAS_PER_SM, false, false, true>(mp, gpool.data(), e.pool_rows); });
-        emu::launch(dim3(k3_blocks), dim3(256), [&] { k_match_slow<false, false, true>(mp, gstack.data(), stack_cap); });
-        G.cursor[rank] = ctrl.cursor;
-        if (ctrl.cursor > G.slab_ids) return -3;
+        Bytes blob(readable + 64, 0);
+        std::memcpy(blob.as<char>(), blob_in, blob_bytes);
+        MatchJob j;
+        j.blob = blob.as<u8>(); j.blob_bytes = blob_bytes; j.readable_bytes = readable; j.offs = offs; j.sel = sel; j.n = n; j.cap = G.slab_ids; j.status = status;
+        j.mode = MatchJob::GATHER; j.gather = &G; j.blocks = G.block.data(); j.rank = rank;
+        MatchGeometry g = e.geometry(false);
+        g.gather_direct = direct != 0;
+        const MatchPlan p = plan_match(g, j, tv.max_depth);
+        MatchBufs m(p);
+        EmuLauncher l;
+        match_pipeline(l, g, j, p, tv, m.scratch());
+        G.cursor[rank] = m.ctrl.as<Ctrl>()->cursor;
+        if (G.cursor[rank] > G.slab_ids) return -3;
     }
-    if (!direct && G.world > 1)
-        emu::launch(dim3(EMU_SMS * 4), dim3(256), [&] {
-            k_gather_push(G.block.data(), rank, G.world, GatherWorld::off_ids, G.off_spans, G.off_index, rank * G.slab_topics, rank * G.slab_ids, n, &G.cursor[rank]);
-        });
+    EmuLauncher l;
+    gather_push(l, G, direct != 0, EMU_SMS, G.block.data(), rank, n, &G.cursor[rank]);
     return 0;
 }
 
@@ -428,10 +330,9 @@ int32_t emu_gather_finish(void* gw, uint32_t rank, uint64_t n, uint32_t new_epoc
     std::vector<unsigned long long*> counts(G.world);
     std::vector<u32*> flags(G.world);
     for (u32 w = 0; w < G.world; ++w) { counts[w] = reinterpret_cast<unsigned long long*>(G.block[w] + G.off_counts); flags[w] = reinterpret_cast<u32*>(G.block[w] + G.off_flags); }
-    u32* my_flags = reinterpret_cast<u32*>(G.block[rank] + G.off_flags);
-    my_flags[32] = 0;                                                                 // the error word
-    emu::launch(dim3(1), dim3(32), [&] { k_gather_finish(counts.data(), flags.data(), my_flags, rank, G.world, n, &G.cursor[rank], G.epoch[rank], my_flags + 32); });
-    return static_cast<int32_t>(my_flags[32]);
+    EmuLauncher l;
+    gather_finish(l, G, G.block[rank], counts.data(), flags.data(), rank, n, &G.cursor[rank], G.epoch[rank]);
+    return static_cast<int32_t>(reinterpret_cast<u32*>(G.block[rank] + G.off_flags)[32]);
 }
 
 // one rank's view of the gathered arrays (gm_gather_get + the copies Engine.gather_result makes)
@@ -441,57 +342,45 @@ void emu_gather_read(void* gw, uint32_t rank, uint64_t* counts, uint32_t* index,
     std::memcpy(counts, b + G.off_counts, static_cast<size_t>(G.world) * 16);
     std::memcpy(index, b + G.off_index, static_cast<size_t>(G.world) * G.slab_topics * 4);
     std::memcpy(spans, b + G.off_spans, static_cast<size_t>(G.world) * G.slab_topics * 8);
-    std::memcpy(ids, b + GatherWorld::off_ids, static_cast<size_t>(G.world) * G.slab_ids * 4);
+    std::memcpy(ids, b + GatherLayout::off_ids, static_cast<size_t>(G.world) * G.slab_ids * 4);
 }
 
-// RetainStorage::get for a batch of filters through k_tokenize -> k_retain_init -> k_retain_round x (depth + 1) -> k_retain_scan -> k_retain_expand
+// RetainStorage::get for a batch of filters through the retained-lookup pipeline, growing the scratch from cap_items / cap_desc
+// like gm_engine::run_retain; *grew = how many times it grew.  Returns 0, -3 with *needed when cap_ids is too small, or
+// GM_ERR_TOO_LARGE when the scratch could not grow any further.
 int32_t emu_retain_match(void* h, const char* blob_in, const uint32_t* offs, uint64_t n64, uint32_t stats_on, uint32_t cap_items, uint32_t cap_desc, gm_span* out_spans,
-                         uint32_t* out_ids, uint64_t cap_ids, uint64_t* needed, int32_t* status, uint64_t* work) {
+                         uint32_t* out_ids, uint64_t cap_ids, uint64_t* needed, int32_t* status, uint64_t* work, uint32_t* grew) {
     EmuEngine& e = *static_cast<EmuEngine*>(h);
     const u32 nq = static_cast<u32>(n64);
     *needed = 0;
+    *grew = 0;
     if (nq == 0) return 0;
     if (!e.prepare(true)) return -7;
     const TrieView tv = e.view();
     const RetainView rv = e.rview();
-    const u32 depth = rv.max_depth, S = depth + 2;
     const u32 blob_bytes = offs[nq];
-    std::vector<u8> blob_store(static_cast<size_t>(blob_bytes) + 64, 0);
-    u8* blob = blob_store.data() + ((16 - (reinterpret_cast<uintptr_t>(blob_store.data()) & 15)) & 15);
-    std::memcpy(blob, blob_in, blob_bytes);
-    std::vector<u32> tok(S > TOK8 ? static_cast<size_t>(S) * nq : 64), meta(nq);
-    std::vector<u32> tok8_store(static_cast<size_t>(nq) * TOK8 + 16);
-    u32* tok8 = tok8_store.data() + ((32 - (reinterpret_cast<uintptr_t>(tok8_store.data()) & 31)) & 31) / 4;
-    struct RCtl { unsigned long long grand; unsigned long long stats[2]; u32 err; u32 pad; u32 n_desc[RQ]; };
-    RCtl ctl{};
-    std::vector<u32> counts(static_cast<size_t>(depth + 3) * RQ + (depth + 3), 0);
-    std::vector<u32> rq(static_cast<size_t>(nq) * 3, 0);
-    u32* qtotal = rq.data(); u32* qbase = qtotal + nq; u32* qcur = qbase + nq;
-    const u32 slice_items = std::max<u32>(1u, cap_items / RQ), slice_desc = std::max<u32>(1u, cap_desc / RQ);
-    std::vector<RTask> front[2] = {std::vector<RTask>(static_cast<size_t>(slice_items) * RQ), std::vector<RTask>(static_cast<size_t>(slice_items) * RQ)};
-    std::vector<RDesc> rdescs(static_cast<size_t>(slice_desc) * RQ);
-    for (u32 i = 0; i < nq; ++i) status[i] = 0x7F7F7F7F;
-    emu::launch(dim3((nq + TOK_THREADS - 1) / TOK_THREADS), dim3(TOK_THREADS), [&] {
-        k_tokenize<false>(blob, blob_bytes, blob_bytes, offs, nullptr, nq, nullptr, tv, S, tok8, tok.data(), meta.data(), status, nullptr, nullptr, 0u, 0u);
-    });
-    RetainParams rp{};
-    rp.v = rv; rp.qtok8 = tok8; rp.qtok = tok.data(); rp.qmeta = meta.data(); rp.nq = nq; rp.tok_levels = S;
-    rp.descs = rdescs.data(); rp.n_desc = ctl.n_desc; rp.cap_items = slice_items; rp.cap_desc = slice_desc;
-    rp.qtotal = qtotal; rp.err = &ctl.err; rp.stats = ctl.stats;
-    emu::launch(dim3((nq + 255) / 256), dim3(256), [&] { if (stats_on) k_retain_init<true>(rp, front[0].data(), &counts[0]); else k_retain_init<false>(rp, front[0].data(), &counts[0]); });
-    const int rgrid = EMU_SMS * GM_RETAIN_CTAS;
-    for (u32 lvl = 0; lvl <= depth; ++lvl)
-        emu::launch(dim3(rgrid), dim3(256), [&] {
-            u32* claim = &counts[static_cast<size_t>(depth + 3) * RQ + lvl];
-            if (stats_on) k_retain_round<true>(rp, front[lvl & 1].data(), &counts[static_cast<size_t>(lvl) * RQ], front[(lvl + 1) & 1].data(), &counts[static_cast<size_t>(lvl + 1) * RQ], claim);
-            else k_retain_round<false>(rp, front[lvl & 1].data(), &counts[static_cast<size_t>(lvl) * RQ], front[(lvl + 1) & 1].data(), &counts[static_cast<size_t>(lvl + 1) * RQ], claim);
-        });
-    emu::launch(dim3(1), dim3(1024), [&] { k_retain_scan(qtotal, nq, qbase, reinterpret_cast<uint2*>(out_spans), &ctl.grand); });
-    emu::launch(dim3(EMU_SMS * 8), dim3(256), [&] { k_retain_expand(rdescs.data(), ctl.n_desc, slice_desc, rv.vals, qbase, qcur, out_ids, cap_ids); });
-    if (work) { work[0] = ctl.stats[0]; work[1] = ctl.stats[1]; }
-    if (ctl.err) return -100 - static_cast<int32_t>(ctl.err);      // scratch overflow: bit 0 tasks, bit 1 descriptors (the engine grows and retries)
-    *needed = ctl.grand;
-    return ctl.grand > cap_ids ? -3 : 0;
+    Bytes blob(static_cast<size_t>(blob_bytes) + 64, 0);
+    std::memcpy(blob.as<char>(), blob_in, blob_bytes);
+    RetainJob j;
+    j.blob = blob.as<u8>(); j.blob_bytes = blob_bytes; j.offs = offs; j.n = nq; j.spans = out_spans; j.ids = out_ids; j.cap_ids = cap_ids; j.status = status;
+    j.stats = stats_on != 0;
+    for (int attempt = 0; attempt < RETAIN_ATTEMPTS; ++attempt) {
+        for (u32 i = 0; i < nq; ++i) status[i] = 0x7F7F7F7F;
+        const RetainPlan p = plan_retain(nq, rv.max_depth, cap_items, cap_desc);
+        Bytes tok(p.tok, 0), tok8(p.tok8, 0), meta(p.meta, 0), rq(p.rq, 0), ctl(p.ctl, 0), front0(p.front, 0), front1(p.front, 0), descs(p.descs, 0);
+        EmuLauncher l;
+        retain_pipeline(l, j, p, tv, rv, {tok.as<u32>(), tok8.as<u32>(), meta.as<u32>(), rq.as<u32>(), ctl.as<RCtl>(), {front0.as<RTask>(), front1.as<RTask>()}, descs.as<RDesc>()},
+                        EMU_SMS);
+        const RCtl& c = *ctl.as<RCtl>();
+        if (c.err == 0) {
+            if (work) { work[0] = c.stats[0]; work[1] = c.stats[1]; }
+            *needed = c.grand;
+            return c.grand > cap_ids ? -3 : 0;
+        }
+        if (!retain_grow(c.err, cap_items, cap_desc)) break;
+        ++*grew;
+    }
+    return GM_ERR_TOO_LARGE;
 }
 
 // gm_relations_expand_device over host arrays (k_relations)

@@ -102,25 +102,18 @@ class Emu:
         spans = np.zeros((n, 2), dtype=np.uint32)
         status = np.zeros(n, dtype=np.int32)
         work = np.zeros(2, dtype=np.uint64)
-        needed = C.c_uint64(0)
-        cap, grew = 1024, 0
+        needed, grew = C.c_uint64(0), C.c_uint32(0)
+        cap = 1024
         blob = np.ascontiguousarray(blob if len(blob) else np.zeros(1, np.uint8))
         while True:
             ids = np.zeros(cap, dtype=np.uint32)
             rc = self.lib.emu_retain_match(self.h, C.c_void_p(blob.ctypes.data), C.c_void_p(offs.ctypes.data), C.c_uint64(n), stats, cap_items, cap_desc, C.c_void_p(spans.ctypes.data), C.c_void_p(ids.ctypes.data),
-                                           C.c_uint64(cap), C.byref(needed), C.c_void_p(status.ctypes.data), C.c_void_p(work.ctypes.data))
+                                           C.c_uint64(cap), C.byref(needed), C.c_void_p(status.ctypes.data), C.c_void_p(work.ctypes.data), C.byref(grew))
             if rc == -3:
                 cap = int(needed.value) + 16
                 continue
-            if rc <= -100:                       # scratch overflow bits: grow like gm_engine::run_retain does
-                err = -rc - 100
-                cap_items *= 4 if err & 1 else 1
-                cap_desc *= 4 if err & 2 else 1
-                grew += 1
-                assert grew < 12
-                continue
             assert rc == 0, rc
-            return MatchResult(spans, ids[:int(needed.value)], status, int(needed.value)), work, grew
+            return MatchResult(spans, ids[:int(needed.value)], status, int(needed.value)), work, int(grew.value)
 
 
 def _canon(want):
@@ -234,7 +227,7 @@ def test_extra_trees_rows_of_the_same_batch(emu):
 def test_retained_pipeline_on_the_emulator_equals_the_oracle(emu, seed):
     """k_tokenize -> k_retain_init -> k_retain_round x (depth + 1) -> k_retain_scan -> k_retain_expand over a random retained
     tree (bulk-built image, then in-place edits), incl. literal '+' / '#' levels that shadow wildcard expansion and a scratch
-    that starts too small (the overflow bits make the caller grow it, as gm_engine::run_retain does)."""
+    that starts too small (the overflow bits make the driver grow it, as gm_engine::run_retain does)."""
     rng = random.Random(seed)
     e, tree = Emu(emu), orc.RetainTree()
     names = []
@@ -622,8 +615,8 @@ def test_workload_generator_shapes_on_parallel_built_tables(emu):
 
 @pytest.mark.parametrize("seed,tiny", [(41, False), (42, True), (43, False)])
 def test_device_image_is_kept_current_by_the_dirty_lists_alone(emu, seed, tiny, monkeypatch):
-    """The kernels read a COPY of every table that only the shipping policy of gm_engine::flush_impl updates (whole table after a
-    re-hash, appended tails, the 32-byte slots the host mirror listed as dirty — tests/native/emu/emu_driver.cpp ImgBuf).  A slot
+    """The kernels read a COPY of every table that only the engine's shipping policy updates (whole table after a re-hash,
+    appended tails, the 32-byte slots the host mirror listed as dirty — rmqtt_b200/csrc/pipeline.h ship(), which gm_engine::flush_impl runs).  A slot
     the mirror changed without listing it would stay stale in the copy and show up as a wrong match.  Rounds of single
     add / remove, a bulk load in between (tables re-hashed), a compaction; subscription trie and retained tree."""
     if tiny:
